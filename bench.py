@@ -18,7 +18,12 @@ every N (golden norms of the oracle, rigid-body modes through the distributed op
 residual of the PCG), and at N = 1 also reports BASELINE configs[2] (Q2 matrix-free), configs[4] (damaged
 reassembly at 10 / 50 / 100 % damage), the FP64 roofline of the element kernels and the CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--size n]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--size n] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes, after the timed steps, what the last of them computed as float64 .npy files: matrix_values
+(the constrained CSR values), cg_x (the PCG iterate, owned dofs) and e2e_du (the Newton increment of the end-to-end leg,
+owned dofs); an output longer than DUMP_ENTRIES allows is a fixed, seeded sample of it.  The inputs are generated from
+fixed seeds, so two builds of the project can be compared output for output.
 """
 from __future__ import annotations
 
@@ -367,6 +372,28 @@ def parity_checks(env, fem, dist, A, form, part, op, n, rows, bvec):
     return out
 
 
+# entries kept per output by --dump-outputs, all ranks together: (4 + 1 + 1) M float64 = 48 MB
+DUMP_ENTRIES = {"matrix_values": 4 << 20, "cg_x": 1 << 20, "e2e_du": 1 << 20}
+
+
+def sample_output(v, k: int, seed: int = 0) -> np.ndarray:
+    """A 1-D tensor as float64 on the host: whole when it has at most `k` entries, else the entries at (up to) `k`
+    sorted indices drawn from `seed`, the same indices on every run with an output of the same length."""
+    import torch
+    n = v.numel()
+    if n > k:
+        idx = np.unique(np.random.default_rng(seed).integers(0, n, size=k))
+        v = v[torch.from_numpy(idx).to(v.device)]
+    return v.detach().to("cpu", torch.float64).numpy()
+
+
+def dump_outputs(path: str, outputs: dict, rank: int, world: int) -> None:
+    """`<path>/<name>.npy` for every output (`<name>_rank<r>.npy` at N > 1)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
 def owned_norms(torch, fem, A, part):
     """(|K|_F^2, trace K) over the owned rows of this rank (device; torch reductions on slices: checker code)."""
     brp, _ = A.block_csr()
@@ -438,6 +465,10 @@ def run_b200(args):
     step_total, _ = env.timed(step, K)
     step_ms = step_total / K
     value = total_dofs / (step_ms * 1e-3) / 1e9
+    outputs = {}
+    if args.dump_outputs:
+        outputs["matrix_values"] = sample_output(A.values, DUMP_ENTRIES["matrix_values"] // world)
+        outputs["cg_x"] = sample_output(xsol[lo:hi], DUMP_ENTRIES["cg_x"] // world)
     asm_total, asm_calls = env.timed(asm, K)
     asm_ms = asm_total / K
     kc = max(1, min(K, 5))
@@ -478,7 +509,10 @@ def run_b200(args):
         op.use("p2p")
 
     # ---- end to end: one Newton linearisation through the public API, host buffers ------------------
-    e2e = e2e_newton(env, fem, dist, form, part, op, A, args, total_dofs)
+    e2e_du, e2e = e2e_newton(env, fem, dist, form, part, op, A, args, total_dofs)
+    if args.dump_outputs:
+        outputs["e2e_du"] = sample_output(e2e_du, DUMP_ENTRIES["e2e_du"] // world)
+        dump_outputs(args.dump_outputs, outputs, rank, world)
 
     # BASELINE configs[4] over the ranks (N > 1; at N = 1 it is part of `extras`)
     c5 = config5_ranks(env, fem, dist, assembly_bytes) if (world > 1 and not args.skip_extras) else None
@@ -567,9 +601,10 @@ def e2e_newton(env, fem, dist, form, part, op, A, args, total_dofs):
     """The same step end to end through the public API with HOST buffers: per step the current iterate u goes up
     from pinned host memory, NewtonSolver.residual (F(u) + lifting) and NewtonSolver.increment (tangent assembly +
     Dirichlet + `cg_iters` PCG iterations) run, and the increment du comes back to pinned host memory.  Geometry,
-    materials and the pattern are resident (uploaded once: they do not change between Newton iterations)."""
+    materials and the pattern are resident (uploaded once: they do not change between Newton iterations).  Returns the
+    host buffer holding the last step's du and the result line's "e2e" entry."""
     torch = env.torch
-    K = max(1, min(args.steps, args.e2e_steps))
+    K = args.e2e_steps or args.steps
     ns = fem.NewtonSolver.__new__(fem.NewtonSolver)          # reuse the bench's matrix / operator (no second 49 GB)
     ns.form, ns.f, ns.A, ns.part = form, None, A, part
     ns.rel_tol, ns.abs_tol, ns.max_iter, ns.convention = 1e-7, 5e-8, 10, "mfem"
@@ -608,15 +643,15 @@ def e2e_newton(env, fem, dist, form, part, op, A, args, total_dofs):
         e2e_step()
     tot, _ = env.timed(lambda: [e2e_step() for _ in range(K)], 1)
     ms = tot / K
-    return {"value": total_dofs / (ms * 1e-3) / 1e9, "unit": UNIT, "ms_per_step": ms, "steps": K,
-            "h2d_bytes_per_step": int(hu.numel() * 8), "d2h_bytes_per_step": int(hdu.numel() * 8),
-            "cpu_cores_bound_to_gpu_numa_node": env.cpu_binding,
-            "du_checksum": float(hdu.abs().sum().item()),
-            "what": "per step and per rank: pinned host u -> device on a copy stream while NewtonSolver.prepare_tangent "
-                    "assembles the tangent (it does not read u: the form is undamaged), NewtonSolver.residual (F(u) + "
-                    "apply_lifting: work the device-timed `value` does not contain), NewtonSolver.increment (Dirichlet "
-                    "rows / columns + Jacobi + PCG), owned du -> pinned host, host waits for it; geometry / materials / "
-                    "pattern resident (constant across Newton iterations)"}
+    return hdu, {"value": total_dofs / (ms * 1e-3) / 1e9, "unit": UNIT, "ms_per_step": ms, "steps": K,
+                 "h2d_bytes_per_step": int(hu.numel() * 8), "d2h_bytes_per_step": int(hdu.numel() * 8),
+                 "cpu_cores_bound_to_gpu_numa_node": env.cpu_binding,
+                 "du_checksum": float(hdu.abs().sum().item()),
+                 "what": "per step and per rank: pinned host u -> device on a copy stream while NewtonSolver.prepare_tangent "
+                         "assembles the tangent (it does not read u: the form is undamaged), NewtonSolver.residual (F(u) + "
+                         "apply_lifting: work the device-timed `value` does not contain), NewtonSolver.increment (Dirichlet "
+                         "rows / columns + Jacobi + PCG), owned du -> pinned host, host waits for it; geometry / materials / "
+                         "pattern resident (constant across Newton iterations)"}
 
 
 def extras(env, fem, peak, args):
@@ -896,7 +931,7 @@ def main():
     ap.add_argument("--cg-iters", type=int, default=25)
     ap.add_argument("--cpu-n", type=int, default=1448, help="cells per side of the CPU sample of --impl reference")
     ap.add_argument("--cpu-baseline-n", type=int, default=1024, help="cells per side of the cpu_baseline leg of the default run")
-    ap.add_argument("--e2e-steps", type=int, default=5)
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the end-to-end leg (default: --steps)")
     ap.add_argument("--transport", default="auto", choices=["auto", "p2p", "nccl"])
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-nccl-compare", action="store_true")
@@ -906,7 +941,13 @@ def main():
                     help="BASELINE config 5 over the ranks instead of the headline step: repeated damaged-tangent reassembly "
                          "(closed form and AD) of 16.8 M P2 elements (nx = 2896)")
     ap.add_argument("--damage-half-width", type=float, default=0.05)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.e2e_steps < 0:
+        ap.error("--steps must be at least 1 and --e2e-steps not negative")
+    if args.dump_outputs and (args.impl == "reference" or args.config5):
+        ap.error("--dump-outputs applies to the B200 step (not --impl reference, not --config5)")
+    sys.dont_write_bytecode = True      # the tree may be read-only: no __pycache__ next to the imported modules
     if args.impl == "reference":
         run_reference(args)
     elif args.config5:
