@@ -23,6 +23,7 @@
 // CGSolver / KSP.
 #include <algorithm>
 
+#include "cg_slots.cuh"
 #include "dist.cuh"
 #include "reduce.cuh"
 
@@ -33,26 +34,6 @@ int pa_apply_launch(const femb200_pa *pa, const double *d_x, double *d_y, const 
 }  // namespace femb
 int64_t pa_num_dofs(const femb200_pa *pa);
 namespace femb {
-
-enum
-{
-   SC_NOM = 0,
-   SC_DEN = 1,
-   SC_BETANOM = 2,
-   SC_R0 = 3,
-   SC_FLAG = 4,
-   SC_ITERS = 5,
-   SC_FINAL = 6,
-   SC_RTOL2 = 7,
-   SC_ATOL2 = 8,
-   SC_RED_NOM = 9,   // local (per-rank) sums written by the vector kernels
-   SC_RED_DEN = 10,
-   SC_RED_BETA = 11,
-   SC_BETA = 12,
-   SC_ALPHA = 13,  // nom / den of the current iteration (cg_core: the x update is deferred to the direction kernel)
-   SC_XPEND = 14,  // 1 while x += alpha d of the current iteration has not been applied yet
-   SC_COUNT = 16
-};
 
 constexpr int kVecThreads = 256;
 

@@ -86,6 +86,19 @@ SIGNATURES = {
                    C.POINTER(C.c_int), vp],
     "femb200_smooth_damage": [vp, vp, vp, i32, f64, vp],
     "femb200_cell_strain_stress": [i32, i64, vp, vp, vp, i32, vp, f64, vp, vp, vp, vp, vp],
+    "femb200_mg_create": [vp, i32, vp, vp, vp, i32, f64, vp, C.POINTER(vp)],
+    "femb200_mg_sizes": [vp, C.POINTER(C.c_int), vp, vp, vp, C.POINTER(i64)],
+    "femb200_mg_galerkin": [vp, vp, i32, vp],
+    "femb200_mg_setup": [vp, vp, vp],
+    "femb200_mg_level_values": [vp, i32, vp, vp],
+    "femb200_mg_coarse_matrix": [vp, vp, vp],
+    "femb200_mg_set_coarse_inverse": [vp, vp, vp],
+    "femb200_mg_restrict": [vp, i32, vp, vp, vp, vp],
+    "femb200_mg_prolong": [vp, i32, vp, vp, vp],
+    "femb200_mg_vcycle": [vp, vp, vp, vp],
+    "femb200_mg_vcycle_timed": [vp, vp, vp, vp, vp],
+    "femb200_pcg_mg": [vp, vp, vp, f64, f64, i32, i32, vp, C.POINTER(C.c_int), C.POINTER(C.c_double),
+                       C.POINTER(C.c_int), vp],
 }
 _SPECIAL = {
     "femb200_version": ([], C.c_int),
@@ -96,6 +109,7 @@ _SPECIAL = {
     "femb200_dist_destroy": ([vp], None),
     "femb200_dist_transport": ([vp], C.c_int),
     "femb200_pa_destroy": ([vp], None),
+    "femb200_mg_destroy": ([vp], None),
 }
 ALL_SYMBOLS = sorted(list(SIGNATURES) + list(_SPECIAL))
 

@@ -331,6 +331,8 @@ class NewtonSolver:
     """The Newton loop around the hot path (mfem::NewtonSolver, M.cc:1531-1549; dolfinx nls::petsc::NewtonSolver,
     F.cc:705-714,869-907).  Per iteration: residual b = F(u) with the Dirichlet lifting (setF, F.cc:817-845), tangent
     J(u) with Dirichlet rows/columns (setJ, F.cc:847-862), Jacobi-PCG solve J du = b, u <- u - du.
+    preconditioner="mg" solves with multigrid-PCG instead (MultigridPreconditioner on `hierarchy`, set up again for
+    every tangent; one GPU only, no `part`).
 
     Both convergence conventions of the reference (doc.tex:2065-2068):
       convention="mfem"     |b| <= max(rel_tol |b_0|, abs_tol), b_0 = the first residual (M.cc:1535-1541);
@@ -343,11 +345,20 @@ class NewtonSolver:
     The tangent is assembled only when an increment is actually computed (after the convergence test), and once
     u carries the boundary values (every iteration after the first) the lifting reduces to set_bc."""
 
+    mg = None   # MultigridPreconditioner with preconditioner="mg"
+
     def __init__(self, form: ElasticityForm, bcs, f=None, rel_tol=1e-7, abs_tol=5e-8, max_iter=10, cg_rel_tol=1e-12,
-                 cg_max_iter=2000, convention: str = "mfem", part=None, transport: str = "auto", group=None):
+                 cg_max_iter=2000, convention: str = "mfem", part=None, transport: str = "auto", group=None,
+                 preconditioner: str = "jacobi", hierarchy=None):
         from . import dist
         if convention not in ("mfem", "dolfinx"):
             raise ValueError("convention must be 'mfem' or 'dolfinx'")
+        if preconditioner not in ("jacobi", "mg"):
+            raise ValueError("preconditioner must be 'jacobi' or 'mg'")
+        if preconditioner == "mg" and part is not None:
+            raise ValueError("the multigrid preconditioner runs on one GPU: it cannot be combined with part=")
+        if preconditioner == "mg" and hierarchy is None:
+            raise ValueError('preconditioner="mg" needs hierarchy= (mesh.lattice_hierarchy / refine_uniform_hierarchy)')
         self.form, self.f = form, to_device(f, np.float64)
         self.rel_tol, self.abs_tol, self.max_iter, self.convention = rel_tol, abs_tol, max_iter, convention
         self.A = create_matrix(form)
@@ -365,15 +376,19 @@ class NewtonSolver:
         self.part = dist.trivial_partition(form.mesh) if part is None else part
         self.cg = dist.DistCG(self.A, self.part, rel_tol=cg_rel_tol, max_iter=cg_max_iter, jacobi=False,
                               transport=transport, group=group)
+        self.cg_rel_tol, self.cg_max_iter = cg_rel_tol, cg_max_iter
+        self.mg = MultigridPreconditioner(self.A, hierarchy) if preconditioner == "mg" else None
         self._lo, self._hi = 2 * self.part.own_lo, 2 * self.part.own_hi
         self._b = torch.empty(self.A.ndofs, dtype=torch.float64, device="cuda")
         self._du = torch.zeros(self.A.ndofs, dtype=torch.float64, device="cuda")
         self._nrm = torch.zeros(1, dtype=torch.float64, device="cuda")
         self._lifted = False          # does u carry the boundary values already?
         self._tangent_ready = False   # A.values holds the unconstrained tangent of the current u
-        self.residual_norms, self.linear_iterations = [], []
+        self.residual_norms, self.linear_iterations, self.linear_converged = [], [], []
 
     def close(self):
+        if self.mg is not None:
+            self.mg.close()
         self.cg.close()
 
     # -- building blocks (one Newton linearisation = residual() + increment()) -----------------
@@ -419,9 +434,19 @@ class NewtonSolver:
         else:
             assemble_matrix(A, form)
         self._tangent_ready = False
+        if self.mg is not None:
+            if fixed_iters:
+                raise ValueError("fixed_iters is not supported with the multigrid preconditioner")
+            self.mg.setup()     # Galerkin levels, smoother and coarse inverse of the new tangent
+            it, _, conv = self.mg.solve(b, self._du, self.cg_rel_tol, 0.0, self.cg_max_iter)
+            self.linear_iterations.append(it)
+            self.linear_converged.append(conv)
+            return self._du
         self.cg.update_preconditioner()
         self.cg.solve(b, self._du, fixed_iters=fixed_iters)
         self.linear_iterations.append(self.cg.iterations)
+        if hasattr(self, "linear_converged"):   # absent on solvers assembled with __new__ (bench.py's end-to-end leg)
+            self.linear_converged.append(self.cg.converged)
         return self._du
 
     def update(self, u: torch.Tensor, du: torch.Tensor) -> torch.Tensor:
@@ -437,6 +462,7 @@ class NewtonSolver:
         A = self.A
         u = torch.zeros(A.ndofs, dtype=torch.float64, device="cuda") if u0 is None else to_device(u0, np.float64).clone()
         self.residual_norms, self.linear_iterations, self.increment_norms = [], [], []
+        self.linear_converged = []
         self._lifted = False
         self.converged = False
         r0 = None
@@ -604,16 +630,191 @@ class PAOperator:
     AssembleDiagonalPA = diagonal
 
 
+class MultigridPreconditioner:
+    """Geometric multigrid V-cycle for an assembled operator `A` (a Matrix with its Dirichlet conditions set) on a
+    nested MeshHierarchy whose finest mesh is A's mesh (mesh.lattice_hierarchy, mesh.refine_uniform_hierarchy).
+
+    Levels: A itself, then the Galerkin operators P^T A P of the coarser meshes, computed on the device by
+    femb200_mg_setup; the hierarchy is cut at the first level with at most `coarse_max` dofs, whose dense inverse
+    (torch.linalg on the device) is the coarse solve.  Smoother: Chebyshev of `degree` on D^-1 A over
+    [lo_frac lambda, lambda], the same before and after the coarse correction, so the V-cycle is symmetric positive
+    definite.  Call setup() after every reassembly of A.values (the V-cycle reads A.values in place)."""
+
+    def __init__(self, A: Matrix, hierarchy, degree: int = 2, coarse_max: int = 4096, lo_frac: float = 0.25):
+        from .mesh import P1
+        _require_cuda()
+        fine = hierarchy.meshes[-1]
+        if fine.ndofs != A.ndofs or fine.etype != A.form.etype:
+            raise ValueError(f"the finest mesh of the hierarchy ({fine.ndofs} dofs) is not the mesh of the operator "
+                             f"({A.ndofs} dofs)")
+        nlev = len(hierarchy.meshes)
+        sizes = [m.ndofs for m in hierarchy.meshes]
+        if nlev < 2:
+            raise ValueError("the hierarchy has no mesh coarser than the fine one")
+        keep = next((k for k in range(nlev - 2, -1, -1) if sizes[k] <= coarse_max), None)
+        if keep is None:
+            raise ValueError(f"the coarsest mesh of the hierarchy has {sizes[0]} dofs, more than coarse_max = {coarse_max}")
+        self.A, self.degree, self.coarse_max = A, int(degree), int(coarse_max)
+        meshes = hierarchy.meshes[keep:]           # coarsest first
+        maps = hierarchy.maps[keep:]
+        fine_marker = A.bc_dev.cpu().numpy() if A.bc_dev is not None else np.zeros(A.ndofs, np.uint8)
+        markers = type(hierarchy)(meshes, maps).markers(fine_marker)
+        # level l = 0 (fine) .. L (coarsest)
+        self.nlevels = len(meshes) - 1
+        self._keep = []                            # device arrays the plans and the handle borrow
+        self._plans = []
+        for k in range(self.nlevels - 1, -1, -1):  # coarse levels 1 .. L
+            m = meshes[k]
+            if m.etype != P1:
+                raise ValueError("coarse levels must be P1")
+            dm = to_device(m.dofmap, np.int32)
+            plan = C.c_void_p()
+            capi.call("femb200_plan_create", capi.P1, m.nnodes, m.ncells, _p(dm), _p(dm), _stream(), C.byref(plan))
+            self._plans.append(plan)
+            self._keep.append(dm)
+        dmaps = [to_device(maps[k], np.int32) for k in range(self.nlevels - 1, -1, -1)]
+        dbcs = [to_device(markers[k], np.uint8) for k in range(self.nlevels - 1, -1, -1)]
+        self._keep += dmaps + dbcs
+        arr = lambda ts: (C.c_void_p * len(ts))(*[t.value if isinstance(t, C.c_void_p) else t.data_ptr() for t in ts])
+        self._handle = C.c_void_p()
+        capi.call("femb200_mg_create", A.plan, self.nlevels, arr(self._plans), arr(dmaps), arr(dbcs), self.degree,
+                  float(lo_frac), _stream(), C.byref(self._handle))
+        self.level_meshes = list(reversed(meshes))  # fine first
+        self._work = None
+        self.ready = False
+
+    def close(self):
+        if getattr(self, "_handle", None) is not None and self._handle.value:
+            capi.lib().femb200_mg_destroy(self._handle)
+            self._handle = C.c_void_p()
+        for p in getattr(self, "_plans", []):
+            if p.value:
+                capi.lib().femb200_plan_destroy(p)
+        self._plans = []
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def handle(self):
+        return self._handle
+
+    def sizes(self):
+        """(dofs per level, nnz per level, lambda per level, device bytes of the handle), fine level first."""
+        L = self.nlevels
+        nl = C.c_int()
+        nd, nz, lam = (C.c_int64 * (L + 1))(), (C.c_int64 * (L + 1))(), (C.c_double * (L + 1))()
+        by = C.c_int64()
+        capi.call("femb200_mg_sizes", self._handle, C.byref(nl), nd, nz, lam, C.byref(by))
+        return list(nd), list(nz), list(lam), by.value
+
+    @property
+    def lambdas(self):
+        return self.sizes()[2]
+
+    def galerkin(self, level: int):
+        """Recompute A_{level+1} = P^T A_level P alone (timing and tests; setup() runs every level)."""
+        capi.call("femb200_mg_galerkin", self._handle, _p(self.A.values), int(level), _stream())
+
+    def setup(self):
+        """Numeric phase: Galerkin cascade, smoother set-up (D^-1, lambda) and the coarse inverse."""
+        capi.call("femb200_mg_setup", self._handle, _p(self.A.values), _stream())
+        self.set_coarse_inverse()
+
+    def set_coarse_inverse(self):
+        Ac = self.coarse_matrix()
+        inv = torch.linalg.inv(Ac)
+        inv = (0.5 * (inv + inv.T)).contiguous()   # exactly symmetric: keeps the V-cycle symmetric
+        capi.call("femb200_mg_set_coarse_inverse", self._handle, _p(inv), _stream())
+        self.ready = True
+
+    def coarse_matrix(self) -> torch.Tensor:
+        n = self.sizes()[0][-1]
+        out = torch.empty((n, n), dtype=torch.float64, device="cuda")
+        capi.call("femb200_mg_coarse_matrix", self._handle, _p(out), _stream())
+        return out
+
+    def level_values(self, level: int) -> torch.Tensor:
+        """CSR values of level 1..L in the pattern of that level's P1 plan (level_csr)."""
+        out = torch.empty(self.sizes()[1][level], dtype=torch.float64, device="cuda")
+        capi.call("femb200_mg_level_values", self._handle, int(level), _p(out), _stream())
+        return out
+
+    def level_csr(self, level: int):
+        """(rowptr int64, colidx int32) device tensors of the scalar CSR pattern of level 1..L."""
+        n = self.sizes()[0][level]
+        nnz = self.sizes()[1][level]
+        rp = torch.empty(n + 1, dtype=torch.int64, device="cuda")
+        ci = torch.empty(nnz, dtype=torch.int32, device="cuda")
+        capi.call("femb200_plan_scalar_csr", self._plans[level - 1], _p(rp), _p(ci), _stream())
+        return rp, ci
+
+    def restrict(self, level: int, b: torch.Tensor, t: torch.Tensor | None = None) -> torch.Tensor:
+        """P^T (b - t) from `level` to level + 1 (t = A x, or None for x = 0)."""
+        out = torch.empty(self.sizes()[0][level + 1], dtype=torch.float64, device="cuda")
+        capi.call("femb200_mg_restrict", self._handle, int(level), _p(b), _p(t), _p(out), _stream())
+        return out
+
+    def prolong(self, level: int, xc: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
+        """x += P xc from level + 1 to `level` (in place)."""
+        capi.call("femb200_mg_prolong", self._handle, int(level), _p(xc), _p(x), _stream())
+        return x
+
+    def apply(self, r: torch.Tensor, z: torch.Tensor | None = None) -> torch.Tensor:
+        """z = B r: one V-cycle."""
+        if not self.ready:
+            raise RuntimeError("MultigridPreconditioner.apply: call setup() first")
+        if z is None:
+            z = torch.empty_like(r)
+        elif z.data_ptr() == r.data_ptr():
+            raise ValueError("MultigridPreconditioner.apply: z must not alias r (the V-cycle reads r after writing z)")
+        capi.call("femb200_mg_vcycle", self._handle, _p(r), _p(z), _stream())
+        return z
+
+    Mult = apply
+
+    def apply_timed(self, r: torch.Tensor, z: torch.Tensor) -> np.ndarray:
+        """One V-cycle with a CUDA event after every launch: (levels, 5) milliseconds per level of its SpMVs,
+        Chebyshev vector passes, restriction, prolongation and coarse GEMV (femb200_mg_vcycle_timed)."""
+        if not self.ready:
+            raise RuntimeError("MultigridPreconditioner.apply_timed: call setup() first")
+        if z.data_ptr() == r.data_ptr():
+            raise ValueError("MultigridPreconditioner.apply_timed: z must not alias r")
+        ms = np.zeros((self.nlevels + 1) * 5)
+        capi.call("femb200_mg_vcycle_timed", self._handle, _p(r), _p(z), ms.ctypes.data_as(C.c_void_p), _stream())
+        return ms.reshape(self.nlevels + 1, 5)
+
+    def solve(self, b: torch.Tensor, x: torch.Tensor, rel_tol: float = 1e-12, abs_tol: float = 0.0, max_iter: int = 2000,
+              check_every: int = 1):
+        """PCG on A with this preconditioner (femb200_pcg_mg): returns (iterations, final <B r, r>^1/2, converged)."""
+        if not self.ready:
+            raise RuntimeError("MultigridPreconditioner.solve: call setup() first")
+        n = self.A.ndofs
+        if self._work is None or self._work.numel() < 4 * n + 64:
+            self._work = torch.empty(4 * n + 64, dtype=torch.float64, device="cuda")
+        it, fn, cv = C.c_int(), C.c_double(), C.c_int()
+        capi.call("femb200_pcg_mg", self._handle, _p(b), _p(x), float(rel_tol), float(abs_tol), int(max_iter),
+                  int(check_every), _p(self._work), C.byref(it), C.byref(fn), C.byref(cv), _stream())
+        return it.value, fn.value, bool(cv.value)
+
+
 class CGSolver:
     """mfem::CGSolver surface (M.cc:1502,1525-1528): SetRelTol / SetAbsTol /
     SetMaxIter / SetOperator / SetPreconditioner / Mult, zero initial guess
-    (iterative_mode = false).  The preconditioner is Jacobi or none."""
+    (iterative_mode = false).  The preconditioner is Jacobi, none, or geometric multigrid
+    (SetPreconditioner("mg", hierarchy=...) or a MultigridPreconditioner)."""
 
-    def __init__(self, rel_tol: float = 1e-12, abs_tol: float = 0.0, max_iter: int = 2000, check_every: int = 25):
+    def __init__(self, rel_tol: float = 1e-12, abs_tol: float = 0.0, max_iter: int = 2000, check_every: int | None = None):
+        """check_every: iterations between host convergence polls; None = 25 for Jacobi / none, 1 for multigrid
+        (a V-cycle queued after convergence is wasted work, a poll costs one synchronisation)."""
         self.rel_tol, self.abs_tol, self.max_iter = rel_tol, abs_tol, max_iter
         self.check_every = check_every
         self.op = None
         self.dinv = None
+        self.mg = None
         self._work = None
         self.iterations, self.final_norm, self.converged = 0, 0.0, False
 
@@ -629,13 +830,31 @@ class CGSolver:
     def SetOperator(self, op):
         self.op = op
         self.dinv = None
+        self.mg = None
 
-    def SetPreconditioner(self, kind: str | None = "jacobi"):
+    def SetPreconditioner(self, kind="jacobi", hierarchy=None, **mg_options):
+        """"jacobi", "none" / None, "mg" (geometric multigrid on `hierarchy`, set up now; call its setup() again
+        after reassembling the operator), or a MultigridPreconditioner of the operator."""
+        self.mg = None
+        if isinstance(kind, MultigridPreconditioner):
+            if kind.A is not self.op:
+                raise ValueError("the multigrid preconditioner was built for another operator")
+            self.dinv, self.mg = None, kind
+            return
         if kind is None or kind == "none":
             self.dinv = None
             return
+        if kind == "mg":
+            if not isinstance(self.op, Matrix):
+                raise ValueError("the multigrid preconditioner needs an assembled operator (Matrix)")
+            if hierarchy is None:
+                raise ValueError('SetPreconditioner("mg") needs hierarchy= (mesh.lattice_hierarchy / refine_uniform_hierarchy)')
+            self.dinv = None
+            self.mg = MultigridPreconditioner(self.op, hierarchy, **mg_options)
+            self.mg.setup()
+            return
         if kind != "jacobi":
-            raise ValueError("only the Jacobi preconditioner is available (BoomerAMG is third party, out of scope)")
+            raise ValueError(f"unknown preconditioner {kind!r}: 'jacobi', 'mg' or 'none'")
         diag = self.op.diagonal()
         self.dinv = torch.empty_like(diag)
         capi.call("femb200_jacobi_setup", diag.numel(), _p(diag), _p(self.dinv), _stream())
@@ -655,6 +874,12 @@ class CGSolver:
         n = b.numel()
         if x is None:
             x = torch.empty_like(b)
+        if self.mg is not None:
+            if fixed_iters:
+                raise ValueError("fixed_iters is not supported with the multigrid preconditioner")
+            self.iterations, self.final_norm, self.converged = self.mg.solve(
+                b, x, self.rel_tol, self.abs_tol, self.max_iter, 1 if self.check_every is None else self.check_every)
+            return x
         if self._work is None or self._work.numel() < 3 * n + 64:
             self._work = torch.empty(3 * n + 64, dtype=torch.float64, device="cuda")
         it, fn, cv = C.c_int(), C.c_double(), C.c_int()
@@ -662,8 +887,9 @@ class CGSolver:
             plan, kind, opp, vals = self.op.plan, capi.OP_CSR, None, _p(self.op.values)
         else:
             plan, kind, opp, vals = None, capi.OP_PA, self.op.handle, None
+        every = 25 if self.check_every is None else self.check_every
         capi.call("femb200_pcg", plan, kind, opp, vals, _p(b), _p(x), n, self.rel_tol, self.abs_tol, self.max_iter,
-                  _p(self.dinv), self.check_every, int(fixed_iters), _p(self._work), C.byref(it), C.byref(fn),
+                  _p(self.dinv), every, int(fixed_iters), _p(self._work), C.byref(it), C.byref(fn),
                   C.byref(cv), _stream())
         self.iterations, self.final_norm, self.converged = it.value, fn.value, bool(cv.value)
         return x

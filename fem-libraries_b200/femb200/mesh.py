@@ -305,6 +305,104 @@ def refine_uniform(mesh: Mesh, levels: int = 1) -> Mesh:
     return mesh
 
 
+@dataclass
+class MeshHierarchy:
+    """Nested meshes for geometric multigrid, coarsest first: meshes[-1] is the finest (the mesh being solved on),
+    every other mesh is P1.  maps[k] ((meshes[k + 1].nnodes, 2) int32) is the transfer from meshes[k + 1] to
+    meshes[k]: per fine node a pair (a, b) of coarse node ids, a == b for a node that coincides with coarse node a
+    (weight 1), otherwise the midpoint of the coarse edge (a, b) (weight 1/2 on each); both components alike.
+    Indexing and len() go over the meshes."""
+    meshes: list
+    maps: list
+
+    def __len__(self) -> int:
+        return len(self.meshes)
+
+    def __getitem__(self, k):
+        return self.meshes[k]
+
+    def markers(self, fine_marker) -> list:
+        """Per-dof Dirichlet markers (uint8) of every mesh, coarsest first, from the finest mesh's marker: a coarse
+        dof is constrained when the fine dof of its coincident node is."""
+        out = [np.asarray(fine_marker, dtype=np.uint8).reshape(-1)]
+        if out[0].size != self.meshes[-1].ndofs:
+            raise ValueError(f"the marker has {out[0].size} entries, the finest mesh {self.meshes[-1].ndofs} dofs")
+        for k in range(len(self.meshes) - 2, -1, -1):
+            co = coincident_nodes(self.maps[k], self.meshes[k].nnodes)
+            m = out[0].reshape(-1, 2)[co].reshape(-1)
+            out.insert(0, np.ascontiguousarray(m))
+        return out
+
+
+def coincident_nodes(tmap: np.ndarray, ncoarse: int) -> np.ndarray:
+    """Fine node that coincides with each coarse node of a transfer map (raises when one has none)."""
+    tmap = np.asarray(tmap)
+    sel = np.nonzero(tmap[:, 0] == tmap[:, 1])[0]
+    co = np.full(ncoarse, -1, dtype=np.int64)
+    co[tmap[sel, 0]] = sel
+    if (co < 0).any():
+        raise ValueError(f"transfer map: {int((co < 0).sum())} coarse nodes have no coincident fine node")
+    return co
+
+
+def _lattice_map(mxf: int, myf: int) -> np.ndarray:
+    """(a, b) of the (mxf x myf)-node lattice halved: node (i, j) -> coarse (i // 2, j // 2) and ((i + 1) // 2,
+    (j + 1) // 2); equal for even (i, j), the two ends of the horizontal, vertical or right-diagonal coarse edge
+    through the node otherwise."""
+    mxc = (mxf - 1) // 2 + 1
+    i, j = np.meshgrid(np.arange(mxf, dtype=np.int64), np.arange(myf, dtype=np.int64), indexing="xy")
+    i, j = i.ravel(), j.ravel()
+    a = (i // 2) + mxc * (j // 2)
+    b = ((i + 1) // 2) + mxc * ((j + 1) // 2)
+    return np.ascontiguousarray(np.stack([a, b], axis=1).astype(np.int32))
+
+
+def lattice_hierarchy(fine: Mesh) -> MeshHierarchy:
+    """Hierarchy of a `structured_triangles` mesh (P1 or P2, any nx x ny, jittered or not): a P2 mesh is coarsened
+    to P1 on the same vertices (its nodes are those of the P1 lattice of 2nx x 2ny cells), then the P1 lattice is
+    halved while both cell counts are even.  Coarse nodes take the coordinates of their coincident fine nodes."""
+    if fine.meta.get("kind") != "structured-tri-right" or fine.etype not in (P1, P2):
+        raise ValueError("lattice_hierarchy: needs a P1 / P2 mesh of structured_triangles")
+    nx, ny = fine.nx, fine.ny
+    meshes, maps = [fine], []
+    sub = 2 if fine.etype == P2 else 1
+    mfx, mfy = sub * nx + 1, sub * ny + 1      # fine node lattice
+    cur = fine
+    while True:
+        if fine.etype == P2 and cur is fine:
+            cx, cy = nx, ny
+        elif cur.nx % 2 == 0 and cur.ny % 2 == 0:
+            cx, cy = cur.nx // 2, cur.ny // 2
+        else:
+            break
+        tmap = _lattice_map(mfx, mfy)
+        c = structured_triangles(cx, cy, order=1)
+        co = coincident_nodes(tmap, c.nnodes)
+        c = Mesh(P1, np.ascontiguousarray(cur.x[co]), c.xdofmap, c.dofmap, cx, cy, dict(c.meta))
+        meshes.insert(0, c)
+        maps.insert(0, tmap)
+        cur, mfx, mfy = c, cx + 1, cy + 1
+    return MeshHierarchy(meshes, maps)
+
+
+def refine_uniform_hierarchy(coarse: Mesh, levels: int) -> MeshHierarchy:
+    """refine_uniform(coarse, 1) `levels` times, keeping every mesh and the transfer maps: the first nv nodes of a
+    refined mesh are the coarse ones, the midpoints follow in sorted-edge order (refine_uniform's numbering), so
+    the finest mesh is refine_uniform(coarse, levels) bit for bit."""
+    meshes, maps = [coarse], []
+    for _ in range(int(levels)):
+        m = meshes[-1]
+        tri = m.xdofmap.astype(np.int64)
+        nv = m.nnodes
+        ea = np.stack([tri[:, [0, 1]], tri[:, [1, 2]], tri[:, [2, 0]]], axis=1).reshape(-1, 2)
+        ukey = np.unique(np.minimum(ea[:, 0], ea[:, 1]) * nv + np.maximum(ea[:, 0], ea[:, 1]))
+        a = np.concatenate([np.arange(nv, dtype=np.int64), ukey // nv])
+        b = np.concatenate([np.arange(nv, dtype=np.int64), ukey % nv])
+        meshes.append(refine_uniform(m, 1))
+        maps.append(np.ascontiguousarray(np.stack([a, b], axis=1).astype(np.int32)))
+    return MeshHierarchy(meshes, maps)
+
+
 def young_from_tags(cell_tags: np.ndarray) -> np.ndarray:
     """E per cell from the physical tag: E_range[tag % 200] (M.cc:1580-1583, F.py:221)."""
     return young_table()[np.asarray(cell_tags, dtype=np.int64) % 200].copy()

@@ -355,6 +355,52 @@ int femb200_cell_strain_stress(int etype, int64_t ncells, const int32_t *d_xdofm
                                const double *d_u, double *d_strain, double *d_stress, void *stream);
 
 /* ------------------------------------------------------------------------
+ * Geometric multigrid preconditioner (assembled CSR operator, single GPU).
+ * Levels 0 (the fine plan, Dirichlet applied through its marker) .. L (coarsest); level l + 1 is a P1 plan.
+ * Transfer map of level l: int32 pair (a, b) of level-(l+1) node ids per level-l node: a == b a coincident
+ * node (weight 1), else the midpoint of the coarse edge (a, b) (weight 1/2 each), both components alike.
+ * P has zero rows for constrained fine dofs and zero columns for constrained coarse dofs (the plans' markers).
+ *   mg_create       borrows the plans (they must outlive the handle); sets the coarse plans' Dirichlet markers
+ *                   from d_coarse_bc[l] (uint8 per dof, NULL: none); validates that the maps are nested (every
+ *                   midpoint on an edge of the coarse pattern, every coarse node and edge hit once);
+ *                   Chebyshev smoother of `degree` on D^-1 A over [lo_frac lambda, lambda].  Synchronises.
+ *   mg_sizes        host: L, and per level 0..L dofs, nnz, lambda (1.1 x 15-step power iteration, after setup)
+ *   mg_galerkin     A_{level+1} = P^T A_level P (gather kernel, write-once) + unit Dirichlet diagonal;
+ *                   level 0 reads d_fine_values (kept by the handle: it must stay valid)
+ *   mg_setup        the numeric phase: every mg_galerkin, D^-1 and lambda per level.  Synchronises.  Re-run
+ *                   after every reassembly of the fine values, then hand in a new coarse inverse.
+ *   mg_level_values copy of the CSR values of level 1..L (the pattern of that level's plan)
+ *   mg_coarse_matrix / mg_set_coarse_inverse: dense row-major image of A_L (n_L^2 doubles), and its inverse
+ *                   (copied into the handle; the V-cycle applies it with a GEMV kernel)
+ *   mg_restrict     d_bc = P^T (d_b - d_t) from level to level + 1 (d_t = A x, or NULL for x = 0)
+ *   mg_prolong      d_x += P d_xc from level + 1 to level
+ *   mg_vcycle       z = B r (z != r): one symmetric V(degree, degree) cycle with an exact coarse solve
+ *   pcg_mg          femb200_pcg with B = mg_vcycle (mfem::CGSolver semantics, nom = <B r, r>); d_work: 4 n + 64
+ *                   doubles; host poll every check_every iterations (<= 0: every one).  Synchronises.
+ * ------------------------------------------------------------------------ */
+typedef struct femb200_mg femb200_mg;
+int femb200_mg_create(const femb200_plan *fine, int nlevels, femb200_plan *const *coarse_plans,
+                      const int32_t *const *d_maps, const uint8_t *const *d_coarse_bc, int degree, double lo_frac,
+                      void *stream, femb200_mg **out);
+void femb200_mg_destroy(femb200_mg *mg);
+int femb200_mg_sizes(const femb200_mg *mg, int *nlevels, int64_t *ndofs, int64_t *nnz, double *lambda,
+                     int64_t *device_bytes);
+int femb200_mg_galerkin(femb200_mg *mg, const double *d_fine_values, int level, void *stream);
+int femb200_mg_setup(femb200_mg *mg, const double *d_fine_values, void *stream);
+int femb200_mg_level_values(const femb200_mg *mg, int level, double *d_out, void *stream);
+int femb200_mg_coarse_matrix(const femb200_mg *mg, double *d_dense, void *stream);
+int femb200_mg_set_coarse_inverse(femb200_mg *mg, const double *d_inv, void *stream);
+int femb200_mg_restrict(const femb200_mg *mg, int level, const double *d_b, const double *d_t, double *d_bc, void *stream);
+int femb200_mg_prolong(const femb200_mg *mg, int level, const double *d_xc, double *d_x, void *stream);
+int femb200_mg_vcycle(femb200_mg *mg, const double *d_r, double *d_z, void *stream);
+/* the same V-cycle with a CUDA event after every launch; ms[(L + 1) * 5] (host) receives per level the milliseconds
+ * of its SpMVs, Chebyshev vector passes, restriction, prolongation and coarse GEMV (event to event, launch gaps
+ * included).  Synchronises. */
+int femb200_mg_vcycle_timed(femb200_mg *mg, const double *d_r, double *d_z, double *ms, void *stream);
+int femb200_pcg_mg(femb200_mg *mg, const double *d_b, double *d_x, double rtol, double atol, int maxit, int check_every,
+                   double *d_work, int *iters, double *final_norm, int *converged, void *stream);
+
+/* ------------------------------------------------------------------------
  * The same entry points under the names SURVEY.md 8b gives the boundary.
  *   create_pattern       = plan_create        (dolfinx create_matrix, F.cc:688)
  *   element_grad_batched = tabulate_tensor_batched in the MFEM layout: elmat column-major,
