@@ -1493,6 +1493,7 @@ static int assemble_matrix_impl(const femb200_plan *p, const double *d_x, int x_
                                 bool dirichlet, double *d_norms = nullptr)
 {
    FEMB_CHECK(p && d_x && d_E && d_values, "assemble_matrix: null argument");
+   FEMB_REFUSE_Q1(p->etype, "assemble_matrix");
    FEMB_CHECK(x_stride == 2 || x_stride == 3, "assemble_matrix: x_stride must be 2 or 3, got %d", x_stride);
    AsmArgs A;
    A.nnodes = p->nnodes, A.nptr = p->nptr, A.vrec = p->vrec, A.frec = p->frec, A.tcnt = p->tcnt, A.thdr = p->thdr, A.perm = p->perm, A.voff = p->voff, A.brp = p->brp;

@@ -55,9 +55,17 @@ static inline int ensure_dynamic_smem(size_t smem)
 }
 
 // ---- element tables --------------------------------------------------------
-__host__ __device__ constexpr int elem_nd(int etype) { return etype == FEMB200_P1 ? 3 : (etype == FEMB200_P2 ? 6 : 9); }
-__host__ __device__ constexpr int elem_nv(int etype) { return etype == FEMB200_Q2 ? 4 : 3; }
+// FEMB200_Q1 is a pattern-only family (coarse multigrid levels): nd = nv = 4, 9 points that no kernel uses
+__host__ __device__ constexpr int elem_nd(int etype)
+{
+   return etype == FEMB200_P1 ? 3 : (etype == FEMB200_P2 ? 6 : (etype == FEMB200_Q1 ? 4 : 9));
+}
+__host__ __device__ constexpr int elem_nv(int etype) { return (etype == FEMB200_Q2 || etype == FEMB200_Q1) ? 4 : 3; }
 __host__ __device__ constexpr int elem_nq(int etype) { return etype == FEMB200_P1 ? 1 : (etype == FEMB200_P2 ? 3 : 9); }
+__host__ __device__ constexpr bool elem_is_triangle(int etype) { return etype == FEMB200_P1 || etype == FEMB200_P2; }
+// every element-level entry point (tabulation, assembly, residual, lifting, PA, output fields) refuses Q1
+#define FEMB_REFUSE_Q1(etype, who) \
+   FEMB_CHECK((etype) != FEMB200_Q1, who ": the Q1 family is pattern only (coarse multigrid levels), it has no element kernel")
 
 // ---- exclusive scans on the device (hand-written, multi-level) --------------
 // out[i] = sum_{k<i} in[k], i in [0, n]; out has n+1 entries.

@@ -293,6 +293,7 @@ extern "C" int femb200_tabulate_tensor_batched(int etype, int64_t ncells, double
                                                double nu, const double *d_dnod, const double *d_u, int variant,
                                                int layout, void *stream)
 {
+   FEMB_REFUSE_Q1(etype, "tabulate");
    FEMB_CHECK(etype >= FEMB200_P1 && etype <= FEMB200_Q2, "tabulate: unknown element family %d", etype);
    FEMB_CHECK(x_stride == 2 || x_stride == 3, "tabulate: x_stride must be 2 or 3, got %d", x_stride);
    FEMB_CHECK(d_A && d_x && d_xdofmap && d_dofmap && d_E, "tabulate: null pointer argument");

@@ -93,6 +93,7 @@ extern "C" int femb200_smooth_damage(const femb200_plan *p, double *d_d, double 
                                      void *stream)
 {
    FEMB_CHECK(p && d_d && d_work, "smooth_damage: null argument");
+   FEMB_REFUSE_Q1(p->etype, "smooth_damage");
    FEMB_CHECK(p->etype == FEMB200_P1, "smooth_damage: the plan must be the P1 (vertex) plan of the triangulation");
    FEMB_CHECK(niter >= 0, "smooth_damage: negative iteration count");
    cudaStream_t st = as_stream(stream);
@@ -111,6 +112,7 @@ extern "C" int femb200_cell_strain_stress(int etype, int64_t ncells, const int32
                                           const double *d_dnod, const double *d_u, double *d_strain, double *d_stress,
                                           void *stream)
 {
+   FEMB_REFUSE_Q1(etype, "cell_strain_stress");
    FEMB_CHECK(etype >= FEMB200_P1 && etype <= FEMB200_Q2, "cell_strain_stress: unknown element family %d", etype);
    FEMB_CHECK(ncells > 0 && d_xdofmap && d_dofmap && d_x && d_u, "cell_strain_stress: null argument");
    FEMB_CHECK(!d_stress || d_E, "cell_strain_stress: the stress needs the Young modulus");

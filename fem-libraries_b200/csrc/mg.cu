@@ -1,20 +1,23 @@
-// mg.cu -- geometric multigrid preconditioner on a nested mesh hierarchy (assembled CSR operators).
+// mg.cu -- geometric multigrid preconditioner on a nested mesh hierarchy.
 //
-// Levels 0 (the operator being solved, Dirichlet rows / columns applied) .. L (coarsest).  Level l + 1 is a P1 space
-// on a mesh whose nodes the fine nodes of level l refer to through one transfer map: an int32 pair (a, b) of coarse
-// node ids per fine node, a == b for a coincident node (weight 1), else the midpoint of the coarse edge (a, b)
-// (weight 1/2 on each).  The same weights act on both components of a node.  P has zero rows for the constrained
-// fine dofs and zero columns for the constrained coarse dofs (the per-dof markers of the level plans).
+// Levels 0 (the operator being solved, Dirichlet rows / columns applied: an assembled CSR plan, or a matrix-free P2 / Q2
+// operator) .. L (coarsest).  Level l + 1 is a P1 or Q1 space on a mesh whose nodes the fine nodes of level l refer to
+// through one transfer map of width 2 or 4 (femb200.h): per fine node the coarse node ids of its coincident node, its
+// coarse edge (a, b) or its coarse quad; each distinct entry weighs 1 / (number of distinct entries).  The same weights
+// act on both components of a node.  P has zero rows for the constrained fine dofs and zero columns for the constrained
+// coarse dofs (the per-dof markers of the levels).  A matrix-free level 0 gets its first coarse operator from the
+// element Galerkin step of pa.cu (a p-coarsening: sum over the cells of P_e^T K_e P_e), without a fine matrix.
 //
 //   Galerkin      A_{l+1} = P^T A_l P, gather form: one group of lanes per coarse node row, one lane per 2x2 output
-//                 block, accumulated in registers and written once; the pattern is the coarse mesh's own P1 pattern
-//                 (every fine pair (i, j) lies in one coarse cell and every non-zero of P for i or j is a vertex of
-//                 that cell), then the coarse Dirichlet rows / columns get a unit diagonal (femb200_apply_dirichlet).
-//                 The fine rows a coarse row reads -- its coincident node and one midpoint per off-diagonal block --
-//                 are resolved once at create time into `slot_fine` (aligned with the coarse bcol).
+//                 block, accumulated in registers and written once; the pattern is the coarse mesh's own P1 / Q1
+//                 pattern (every fine pair (i, j) lies in one coarse cell and every non-zero of P for i or j is a vertex
+//                 of that cell), then the coarse Dirichlet rows / columns get a unit diagonal (femb200_apply_dirichlet).
+//                 The fine rows a coarse row reads -- its coincident node and one midpoint or quad centre per
+//                 off-diagonal block -- are resolved once at create time into `slot_fine` (aligned with the coarse bcol).
 //   smoother      Chebyshev of degree k on D^-1 A over [lo lambda, lambda], lambda = 1.1 x a 15-step power iteration
 //                 from a fixed seed; the same polynomial before and after the coarse correction (symmetric V(k,k)).
-//                 A d goes through femb200_spmv; the recurrence r -= D^-1 A d, d = c1 d + c2 r, x += d is one pass.
+//                 A d goes through femb200_spmv (the matrix-free apply on a matrix-free level 0); the recurrence
+//                 r -= D^-1 A d, d = c1 d + c2 r, x += d is one pass.
 //   transfers     r_c = P^T (b - A x) in gather form (one thread per coarse node), x += P x_c (one per fine node).
 //   coarsest      x = C b with C the dense inverse handed in by the caller (femb200_mg_set_coarse_inverse).
 //   PCG           mfem::CGSolver semantics with B = one V-cycle (nom = <B r, r>), the scalar kernels of cg.cu.
@@ -40,16 +43,17 @@ constexpr uint64_t kPowerSeed = 0x6d67706f77657231ull;
 
 struct MgLevel
 {
-   femb200_plan *plan = nullptr;  // borrowed; level 0: the fine plan
+   femb200_plan *plan = nullptr;     // borrowed; level 0: the fine plan, or null for a matrix-free level 0
+   const femb200_pa *pa = nullptr;   // borrowed; level 0 of a matrix-free operator
    int64_t nnodes = 0, n = 0;
-   const double *values = nullptr;  // level 0: borrowed from setup; else = own_values
+   const double *values = nullptr;  // level 0: borrowed from setup (null when matrix-free); else = own_values
    double *own_values = nullptr;    // [nnz]
    double *dinv = nullptr, *r = nullptr, *d = nullptr, *t = nullptr;  // [n]
    double *b = nullptr, *x = nullptr;                                   // [n], levels >= 1
    double lambda = 0.;
    double inv_theta = 0., c1[kMaxDegree] = {}, c2[kMaxDegree] = {};
    // transfer to level + 1
-   int2 *map = nullptr;          // [nnodes]
+   int32_t *map = nullptr;        // [nnodes][width]
    int32_t *slot_fine = nullptr;  // [nnzb of level + 1]
    int group = 0;                 // lanes per coarse row of the Galerkin kernel (level + 1 rows)
 };
@@ -70,54 +74,118 @@ __device__ __forceinline__ int find_col(const int32_t *__restrict__ bcol, int64_
    return -1;
 }
 
-// slot_fine[s] = the fine node whose coarse row / column pair is the block slot s of the coarse pattern: the coincident
-// node of the diagonal block, the midpoint of the edge of an off-diagonal one.  err: 1 map entry out of range, 2 a
-// midpoint whose edge is not in the coarse pattern, 3 two fine nodes on one coarse slot, 4 a coarse slot without one.
-__global__ void mg_slots_kernel(int64_t nf, const int2 *__restrict__ map, int64_t nc, const int64_t *__restrict__ cbrp,
+// One row of a transfer map of width W (2 or 4): the coarse node ids of a fine node.
+template <int W>
+struct MapRow
+{
+   int m[W];
+};
+
+template <int W>
+__device__ __forceinline__ MapRow<W> load_map(const int32_t *__restrict__ map, int64_t i)
+{
+   MapRow<W> r;
+   if constexpr (W == 2)
+   {
+      const int2 v = reinterpret_cast<const int2 *>(map)[i];
+      r.m[0] = v.x, r.m[1] = v.y;
+   }
+   else
+   {
+      const int4 v = reinterpret_cast<const int4 *>(map)[i];
+      r.m[0] = v.x, r.m[1] = v.y, r.m[2] = v.z, r.m[3] = v.w;
+   }
+   return r;
+}
+
+// weight of coarse node J in the interpolation of the fine node: 1 / (number of distinct entries) when J is one of them.
+// Pairs: 1 for a coincident node, 1/2 for a midpoint.  Width 4 (rows validated by mg_slots_kernel): (a, a, a, a) 1,
+// (a, b, a, b) 1/2, a quad centre 1/4.
+template <int W>
+__device__ __forceinline__ double map_weight(const MapRow<W> &r, int J)
+{
+   if constexpr (W == 2)
+      return 0.5 * ((r.m[0] == J) + (r.m[1] == J));
+   else
+   {
+      if (r.m[0] != J && r.m[1] != J && r.m[2] != J && r.m[3] != J) return 0.;
+      return r.m[0] == r.m[3] ? 1. : (r.m[0] == r.m[2] ? 0.5 : 0.25);
+   }
+}
+
+// slot_fine[s] = the fine node whose coarse pairs include the block slot s of the coarse pattern: entry k of its map row
+// and its partner W - 1 - k name the slot (map[k], map[W-1-k]): the diagonal block of a coincident node, the two blocks
+// of the edge of a midpoint, the four blocks of the two diagonals of a quad centre.  err: 1 map entry out of range,
+// 2 a pair that is not in the coarse pattern, 3 two fine nodes on one coarse slot, 4 a coarse slot without one,
+// 5 a width-4 row that is none of (a, a, a, a), (a, b, a, b), four distinct nodes.
+template <int W>
+__global__ void mg_slots_kernel(int64_t nf, const int32_t *__restrict__ map, int64_t nc, const int64_t *__restrict__ cbrp,
                                 const int32_t *__restrict__ cbcol, int32_t *__restrict__ slot_fine, int *__restrict__ err)
 {
    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
    if (i >= nf) return;
-   const int2 ab = map[i];
-   if (ab.x < 0 || ab.y < 0 || ab.x >= nc || ab.y >= nc)
+   const MapRow<W> r = load_map<W>(map, i);
+#pragma unroll
+   for (int k = 0; k < W; ++k)
+      if (r.m[k] < 0 || r.m[k] >= nc)
+      {
+         *err = 1;
+         return;
+      }
+   if constexpr (W == 4)
    {
-      *err = 1;
-      return;
+      const int *m = r.m;
+      const bool co = m[0] == m[1] && m[1] == m[2] && m[2] == m[3];
+      const bool edge = m[0] == m[2] && m[1] == m[3] && m[0] != m[1];
+      const bool quad = m[0] != m[1] && m[0] != m[2] && m[0] != m[3] && m[1] != m[2] && m[1] != m[3] && m[2] != m[3];
+      if (!co && !edge && !quad)
+      {
+         *err = 5;
+         return;
+      }
    }
-   const int64_t ba = cbrp[ab.x], bb = cbrp[ab.y];
-   const int ka = find_col(cbcol, ba, (int)(cbrp[ab.x + 1] - ba), ab.y);
-   const int kb = find_col(cbcol, bb, (int)(cbrp[ab.y + 1] - bb), ab.x);
-   if (ka < 0 || kb < 0)
+#pragma unroll
+   for (int k = 0; k < W; ++k)
    {
-      *err = 2;
-      return;
+      const int a = r.m[k], b = r.m[W - 1 - k];
+      const int64_t ba = cbrp[a];
+      const int ka = find_col(cbcol, ba, (int)(cbrp[a + 1] - ba), b);
+      if (ka < 0)
+      {
+         *err = 2;
+         return;
+      }
+      slot_fine[ba + ka] = (int32_t)i;
    }
-   slot_fine[ba + ka] = (int32_t)i;
-   slot_fine[bb + kb] = (int32_t)i;
 }
 
-__global__ void mg_slots_check_kernel(int64_t nf, const int2 *__restrict__ map, const int64_t *__restrict__ cbrp,
+template <int W>
+__global__ void mg_slots_check_kernel(int64_t nf, const int32_t *__restrict__ map, const int64_t *__restrict__ cbrp,
                                       const int32_t *__restrict__ cbcol, const int32_t *__restrict__ slot_fine,
                                       int64_t nnzb_c, int *__restrict__ err)
 {
    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
    if (i < nnzb_c && slot_fine[i] < 0) *err = 4;
-   if (i >= nf || *err == 1 || *err == 2) return;
-   const int2 ab = map[i];
-   const int64_t ba = cbrp[ab.x];
-   const int ka = find_col(cbcol, ba, (int)(cbrp[ab.x + 1] - ba), ab.y);
-   if (slot_fine[ba + ka] != (int32_t)i) *err = 3;
+   if (i >= nf || *err == 1 || *err == 2 || *err == 5) return;
+   const MapRow<W> r = load_map<W>(map, i);
+#pragma unroll
+   for (int k = 0; k < W; ++k)
+   {
+      const int64_t ba = cbrp[r.m[k]];
+      const int ka = find_col(cbcol, ba, (int)(cbrp[r.m[k] + 1] - ba), r.m[W - 1 - k]);
+      if (slot_fine[ba + ka] != (int32_t)i) *err = 3;
+   }
 }
 
 // A_c = P^T A P.  G lanes per coarse node row I (G >= its block degree); lane k owns the output block (I, J = bcol[k])
 // and scans the fine rows of the row (slot_fine) and their fine blocks in a fixed order, accumulating the fine blocks
 // (i, j) whose column node j has a weight on J.  Values layout (femb200.h): A[2i + ci, 2j + cj] at
 // 4 brp[i] + 2 ci deg(i) + 2 (slot of j) + cj.
-template <int G>
+template <int G, int W>
 __global__ void __launch_bounds__(kMgThreads)
 mg_rap_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *__restrict__ cbcol,
               const int32_t *__restrict__ slot_fine, const int64_t *__restrict__ fbrp, const int32_t *__restrict__ fbcol,
-              const double *__restrict__ fval, const int2 *__restrict__ map, const uint8_t *__restrict__ fbc,
+              const double *__restrict__ fval, const int32_t *__restrict__ map, const uint8_t *__restrict__ fbc,
               double *__restrict__ cval)
 {
    const int64_t I = ((int64_t)blockIdx.x * kMgThreads + threadIdx.x) / G;
@@ -130,7 +198,7 @@ mg_rap_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *__res
    for (int p = 0; p < nb; ++p)
    {
       const int64_t i = slot_fine[cb + p];
-      const double wi = cbcol[cb + p] == (int32_t)I ? 1. : 0.5;
+      const double wi = map_weight<W>(load_map<W>(map, i), (int)I);
       const double wi0 = (fbc && fbc[2 * i]) ? 0. : wi, wi1 = (fbc && fbc[2 * i + 1]) ? 0. : wi;
       const int64_t fb = fbrp[i];
       const int fdeg = (int)(fbrp[i + 1] - fb);
@@ -138,10 +206,8 @@ mg_rap_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *__res
       for (int q = 0; q < fdeg; ++q)
       {
          const int64_t j = fbcol[fb + q];
-         const int2 ab = map[j];
-         const int hits = (ab.x == J) + (ab.y == J);
-         if (hits == 0) continue;
-         const double wj = 0.5 * hits;
+         const double wj = map_weight<W>(load_map<W>(map, j), J);
+         if (wj == 0.) continue;
          const double wj0 = (fbc && fbc[2 * j]) ? 0. : wj, wj1 = (fbc && fbc[2 * j + 1]) ? 0. : wj;
          const double2 v0 = *reinterpret_cast<const double2 *>(row0 + 2 * q);
          const double2 v1 = *reinterpret_cast<const double2 *>(row1 + 2 * q);
@@ -159,9 +225,10 @@ mg_rap_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *__res
 }
 
 // bc[2I + c] = (P^T (b - t))[2I + c], one thread per coarse node; t = A x or null (x = 0)
+template <int W>
 __global__ void __launch_bounds__(kMgThreads)
-mg_restrict_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *__restrict__ cbcol,
-                   const int32_t *__restrict__ slot_fine, const uint8_t *__restrict__ fbc, const uint8_t *__restrict__ cbc,
+mg_restrict_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *__restrict__ slot_fine,
+                   const int32_t *__restrict__ map, const uint8_t *__restrict__ fbc, const uint8_t *__restrict__ cbc,
                    const double2 *__restrict__ b, const double2 *__restrict__ t, double2 *__restrict__ out)
 {
    const int64_t I = (int64_t)blockIdx.x * kMgThreads + threadIdx.x;
@@ -172,7 +239,7 @@ mg_restrict_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *
    for (int p = 0; p < nb; ++p)
    {
       const int64_t i = slot_fine[cb + p];
-      const double w = cbcol[cb + p] == (int32_t)I ? 1. : 0.5;
+      const double w = map_weight<W>(load_map<W>(map, i), (int)I);
       const double w0 = (fbc && fbc[2 * i]) ? 0. : w, w1 = (fbc && fbc[2 * i + 1]) ? 0. : w;
       const double2 bi = b[i];
       const double2 ti = t ? t[i] : make_double2(0., 0.);
@@ -187,36 +254,43 @@ mg_restrict_kernel(int64_t nc, const int64_t *__restrict__ cbrp, const int32_t *
    out[I] = make_double2(s0, s1);
 }
 
-// x += P x_c, one thread per fine node
+// x += P x_c, one thread per fine node: (P x_c)_i summed over the distinct coarse nodes in ascending id, as a CSR
+// product with sorted columns does (the weights 1, 1/2, 1/4 make every product exact)
+template <int W>
 __global__ void __launch_bounds__(kMgThreads)
-mg_prolong_kernel(int64_t nf, const int2 *__restrict__ map, const uint8_t *__restrict__ fbc, const uint8_t *__restrict__ cbc,
-                  const double *__restrict__ xc, double *__restrict__ x)
+mg_prolong_kernel(int64_t nf, const int32_t *__restrict__ map, const uint8_t *__restrict__ fbc,
+                  const uint8_t *__restrict__ cbc, const double *__restrict__ xc, double *__restrict__ x)
 {
    const int64_t i = (int64_t)blockIdx.x * kMgThreads + threadIdx.x;
    if (i >= nf) return;
-   const int2 ab = map[i];
+   const MapRow<W> r = load_map<W>(map, i);
+   int cn[W], nd = 0;  // distinct entries, ascending
+#pragma unroll
+   for (int k = 0; k < W; ++k)
+   {
+      const int v = r.m[k];
+      bool seen = false;
+      for (int t = 0; t < nd; ++t) seen = seen || cn[t] == v;
+      if (seen) continue;
+      int p = nd++;
+      for (; p > 0 && cn[p - 1] > v; --p) cn[p] = cn[p - 1];
+      cn[p] = v;
+   }
+   const double w = nd == 1 ? 1. : (nd == 2 ? 0.5 : 0.25);
 #pragma unroll
    for (int c = 0; c < 2; ++c)
    {
       if (fbc && fbc[2 * i + c]) continue;
-      const bool ma = !(cbc && cbc[2 * ab.x + c]), mb = !(cbc && cbc[2 * ab.y + c]);
-      double v;
-      if (ab.x == ab.y)
+      double v = 0.;
+      bool any = false;
+      for (int t = 0; t < nd; ++t)
       {
-         if (!ma) continue;
-         v = xc[2 * ab.x + c];
+         if (cbc && cbc[2 * cn[t] + c]) continue;
+         const double s = nd == 1 ? xc[2 * cn[t] + c] : __dmul_rn(w, xc[2 * cn[t] + c]);
+         v = t == 0 ? s : __dadd_rn(v, s);
+         any = true;
       }
-      else
-      {
-         // (P x_c)_i summed in ascending column order, as a CSR product does; 0.5 x is exact
-         const int lo = min(ab.x, ab.y), hi = max(ab.x, ab.y);
-         const bool mlo = lo == ab.x ? ma : mb, mhi = lo == ab.x ? mb : ma;
-         v = 0.;
-         if (mlo) v = __dmul_rn(0.5, xc[2 * lo + c]);
-         if (mhi) v = __dadd_rn(v, __dmul_rn(0.5, xc[2 * hi + c]));
-         if (!mlo && !mhi) continue;
-      }
-      x[2 * i + c] = __dadd_rn(x[2 * i + c], v);
+      if (any) x[2 * i + c] = __dadd_rn(x[2 * i + c], v);
    }
 }
 
@@ -415,6 +489,7 @@ int mg_alloc(T **p, int64_t count, size_t *bytes)
 struct femb200_mg
 {
    std::vector<femb::MgLevel> lev;  // 0 .. L
+   int width = 2;                   // transfer map width (2 pairs, 4 with quad centres)
    int degree = 2;
    double lo_frac = 0.25;
    double *cinv = nullptr;  // [nc x nc]
@@ -423,6 +498,16 @@ struct femb200_mg
    bool have_values = false, have_inverse = false;
    size_t bytes = 0;
 };
+
+namespace femb {
+int pa_apply_launch(const femb200_pa *pa, const double *d_x, double *d_y, const double *d_flag, double *d_dot_out,
+                    cudaStream_t st, bool accumulate);
+int pa_mg_info(const femb200_pa *pa, int *etype, int64_t *nnodes, int64_t *ncells);
+const uint8_t *pa_dirichlet_marker(const femb200_pa *pa);
+int pa_check_pcoarsening(const femb200_pa *pa, const femb200_plan *coarse, const int32_t *d_map, int width, int *d_err,
+                         cudaStream_t st);
+int pa_element_galerkin(const femb200_pa *pa, const femb200_plan *coarse, double *d_values, cudaStream_t st);
+}  // namespace femb
 
 using namespace femb;
 
@@ -441,16 +526,44 @@ static void mg_free(femb200_mg *mg)
 
 extern "C" void femb200_mg_destroy(femb200_mg *mg) { mg_free(mg); }
 
-static int mg_create_impl(femb200_mg *mg, const femb200_plan *fine, int nlevels, femb200_plan *const *coarse_plans,
+// Dirichlet marker of a level, read at every launch: femb200_plan_set_dirichlet / femb200_pa_set_dirichlet replace it
+static const uint8_t *level_bc(const MgLevel &v) { return v.pa ? pa_dirichlet_marker(v.pa) : v.plan->bc; }
+
+// y = A_l x: the level's SpMV, or the matrix-free apply of level 0
+static int mg_apply(const femb200_mg *mg, int l, const double *x, double *y, cudaStream_t st)
+{
+   const MgLevel &v = mg->lev[l];
+   if (v.pa) return pa_apply_launch(v.pa, x, y, nullptr, nullptr, st, false);
+   return femb200_spmv(v.plan, v.values, x, y, st);
+}
+
+static int mg_create_impl(femb200_mg *mg, int op_kind, const void *fine_op, int nlevels, femb200_plan *const *coarse_plans,
                           const int32_t *const *d_maps, const uint8_t *const *d_coarse_bc, cudaStream_t st)
 {
    mg->lev.resize(nlevels + 1);
    for (int l = 0; l <= nlevels; ++l)
    {
       MgLevel &v = mg->lev[l];
-      v.plan = l == 0 ? const_cast<femb200_plan *>(fine) : coarse_plans[l - 1];
+      if (l == 0 && op_kind == FEMB200_OP_PA)
+      {
+         v.pa = static_cast<const femb200_pa *>(fine_op);
+         int et = 0;
+         int64_t nn = 0, ncell = 0;
+         if (int rc = pa_mg_info(v.pa, &et, &nn, &ncell)) return rc;
+         FEMB_CHECK(et == FEMB200_P2 || et == FEMB200_Q2,
+                    "mg_create: a matrix-free fine level must be P2 or Q2, its first coarse level a p-coarsening (P2 -> P1 "
+                    "or Q2 -> Q1 on the same cells)");
+         v.nnodes = nn, v.n = 2 * nn;
+         continue;
+      }
+      v.plan = l == 0 ? const_cast<femb200_plan *>(static_cast<const femb200_plan *>(fine_op)) : coarse_plans[l - 1];
       FEMB_CHECK(v.plan, "mg_create: null plan of level %d", l);
-      if (l > 0) FEMB_CHECK(v.plan->etype == FEMB200_P1, "mg_create: coarse level %d is not a P1 plan", l);
+      if (l > 0)
+      {
+         const int want = mg->width == 2 ? FEMB200_P1 : FEMB200_Q1;
+         FEMB_CHECK(v.plan->etype == want, "mg_create: coarse level %d is not a %s plan (transfer maps of width %d)", l,
+                    want == FEMB200_P1 ? "P1" : "Q1", mg->width);
+      }
       v.nnodes = v.plan->nnodes, v.n = 2 * v.nnodes;
    }
    const int64_t nc = mg->lev[nlevels].n;
@@ -460,6 +573,7 @@ static int mg_create_impl(femb200_mg *mg, const femb200_plan *fine, int nlevels,
        mg_alloc(&mg->cinv, nc * nc, &mg->bytes))
       return 1;
    FEMB_CUDA(cudaMemsetAsync(mg->err, 0, sizeof(int), st));
+   const int W = mg->width;
    for (int l = 0; l <= nlevels; ++l)
    {
       MgLevel &v = mg->lev[l];
@@ -485,37 +599,51 @@ static int mg_create_impl(femb200_mg *mg, const femb200_plan *fine, int nlevels,
       FEMB_CHECK(deg <= 32, "mg_create: coarse level %d has a node with %d neighbours (at most 32)", l + 1, deg);
       v.group = deg <= 8 ? 8 : (deg <= 16 ? 16 : 32);
       FEMB_CHECK(d_maps && d_maps[l], "mg_create: null transfer map of level %d", l);
-      if (mg_alloc(&v.map, v.nnodes, &mg->bytes) || mg_alloc(&v.slot_fine, cp->nnzb, &mg->bytes)) return 1;
-      FEMB_CUDA(cudaMemcpyAsync(v.map, d_maps[l], (size_t)v.nnodes * sizeof(int2), cudaMemcpyDeviceToDevice, st));
+      if (mg_alloc(&v.map, v.nnodes * W, &mg->bytes) || mg_alloc(&v.slot_fine, cp->nnzb, &mg->bytes)) return 1;
+      FEMB_CUDA(cudaMemcpyAsync(v.map, d_maps[l], (size_t)v.nnodes * W * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
       FEMB_CUDA(cudaMemsetAsync(v.slot_fine, 0xff, (size_t)cp->nnzb * sizeof(int32_t), st));
-      mg_slots_kernel<<<(unsigned)cdiv(v.nnodes, 256), 256, 0, st>>>(v.nnodes, v.map, cp->nnodes, cp->brp, cp->bcol,
-                                                                     v.slot_fine, mg->err);
-      FEMB_LAUNCH_CHECK();
-      mg_slots_check_kernel<<<(unsigned)cdiv(std::max<int64_t>(v.nnodes, cp->nnzb), 256), 256, 0, st>>>(
-          v.nnodes, v.map, cp->brp, cp->bcol, v.slot_fine, cp->nnzb, mg->err);
+      const unsigned g1 = (unsigned)cdiv(v.nnodes, 256), g2 = (unsigned)cdiv(std::max<int64_t>(v.nnodes, cp->nnzb), 256);
+      if (W == 2)
+      {
+         mg_slots_kernel<2><<<g1, 256, 0, st>>>(v.nnodes, v.map, cp->nnodes, cp->brp, cp->bcol, v.slot_fine, mg->err);
+         FEMB_LAUNCH_CHECK();
+         mg_slots_check_kernel<2><<<g2, 256, 0, st>>>(v.nnodes, v.map, cp->brp, cp->bcol, v.slot_fine, cp->nnzb, mg->err);
+      }
+      else
+      {
+         mg_slots_kernel<4><<<g1, 256, 0, st>>>(v.nnodes, v.map, cp->nnodes, cp->brp, cp->bcol, v.slot_fine, mg->err);
+         FEMB_LAUNCH_CHECK();
+         mg_slots_check_kernel<4><<<g2, 256, 0, st>>>(v.nnodes, v.map, cp->brp, cp->bcol, v.slot_fine, cp->nnzb, mg->err);
+      }
       FEMB_LAUNCH_CHECK();
       int herr = 0;
       FEMB_CUDA(cudaMemcpyAsync(&herr, mg->err, sizeof(int), cudaMemcpyDeviceToHost, st));
       FEMB_CUDA(cudaStreamSynchronize(st));
-      static const char *what[] = {"", "a coarse node id is out of range", "a midpoint lies on no edge of the coarse mesh",
-                                   "two fine nodes map to the same coarse node or edge",
-                                   "a coarse node or edge has no fine node"};
-      FEMB_CHECK(herr == 0, "mg_create: level %d -> %d is not a nested hierarchy: %s", l, l + 1, what[herr & 7]);
+      static const char *what[] = {"", "a coarse node id is out of range",
+                                   "a fine node's coarse pair (edge or quad diagonal) is not in the coarse pattern",
+                                   "two fine nodes map to the same coarse node, edge or quad",
+                                   "a coarse node, edge or quad has no fine node",
+                                   "a width-4 map row is none of (a, a, a, a), (a, b, a, b), four distinct nodes"};
+      FEMB_CHECK(herr == 0, "mg_create: level %d -> %d is not a nested hierarchy: %s", l, l + 1, what[herr % 6]);
+      if (l == 0 && v.pa)
+         if (int rc = pa_check_pcoarsening(v.pa, cp, v.map, W, mg->err, st)) return rc;
    }
    return 0;
 }
 
-extern "C" int femb200_mg_create(const femb200_plan *fine, int nlevels, femb200_plan *const *coarse_plans,
-                                 const int32_t *const *d_maps, const uint8_t *const *d_coarse_bc, int degree,
-                                 double lo_frac, void *stream, femb200_mg **out)
+extern "C" int femb200_mg_create_op(int op_kind, const void *fine_op, int nlevels, femb200_plan *const *coarse_plans,
+                                    const int32_t *const *d_maps, int map_width, const uint8_t *const *d_coarse_bc,
+                                    int degree, double lo_frac, void *stream, femb200_mg **out)
 {
-   FEMB_CHECK(out && fine && nlevels >= 1 && coarse_plans && d_maps, "mg_create: bad argument");
+   FEMB_CHECK(out && fine_op && nlevels >= 1 && coarse_plans && d_maps, "mg_create: bad argument");
+   FEMB_CHECK(op_kind == FEMB200_OP_CSR || op_kind == FEMB200_OP_PA, "mg_create: unknown operator kind %d", op_kind);
+   FEMB_CHECK(map_width == 2 || map_width == 4, "mg_create: transfer map width %d (2 or 4)", map_width);
    FEMB_CHECK(degree >= 1 && degree <= kMaxDegree, "mg_create: Chebyshev degree %d outside [1, %d]", degree, kMaxDegree);
    FEMB_CHECK(lo_frac > 0. && lo_frac < 1., "mg_create: lower interval fraction %g outside (0, 1)", lo_frac);
    *out = nullptr;
    femb200_mg *mg = new femb200_mg();
-   mg->degree = degree, mg->lo_frac = lo_frac;
-   if (int rc = mg_create_impl(mg, fine, nlevels, coarse_plans, d_maps, d_coarse_bc, as_stream(stream)))
+   mg->width = map_width, mg->degree = degree, mg->lo_frac = lo_frac;
+   if (int rc = mg_create_impl(mg, op_kind, fine_op, nlevels, coarse_plans, d_maps, d_coarse_bc, as_stream(stream)))
    {
       cudaStreamSynchronize(as_stream(stream));
       mg_free(mg);
@@ -523,6 +651,14 @@ extern "C" int femb200_mg_create(const femb200_plan *fine, int nlevels, femb200_
    }
    *out = mg;
    return 0;
+}
+
+extern "C" int femb200_mg_create(const femb200_plan *fine, int nlevels, femb200_plan *const *coarse_plans,
+                                 const int32_t *const *d_maps, const uint8_t *const *d_coarse_bc, int degree,
+                                 double lo_frac, void *stream, femb200_mg **out)
+{
+   return femb200_mg_create_op(FEMB200_OP_CSR, fine, nlevels, coarse_plans, d_maps, 2, d_coarse_bc, degree, lo_frac,
+                               stream, out);
 }
 
 extern "C" int femb200_mg_sizes(const femb200_mg *mg, int *nlevels, int64_t *ndofs, int64_t *nnz, double *lambda,
@@ -534,11 +670,32 @@ extern "C" int femb200_mg_sizes(const femb200_mg *mg, int *nlevels, int64_t *ndo
    for (int l = 0; l <= L; ++l)
    {
       if (ndofs) ndofs[l] = mg->lev[l].n;
-      if (nnz) nnz[l] = 4 * mg->lev[l].plan->nnzb;
+      if (nnz) nnz[l] = mg->lev[l].plan ? 4 * mg->lev[l].plan->nnzb : 0;
       if (lambda) lambda[l] = mg->lev[l].lambda;
    }
    if (device_bytes) *device_bytes = (int64_t)mg->bytes;
    return 0;
+}
+
+template <int W>
+static void mg_rap_launch(const MgLevel &f, const MgLevel &c, cudaStream_t st)
+{
+   const femb200_plan *fp = f.plan, *cp = c.plan;
+   const unsigned grid = (unsigned)cdiv(cp->nnodes * f.group, kMgThreads);
+   switch (f.group)
+   {
+   case 8:
+      mg_rap_kernel<8, W><<<grid, kMgThreads, 0, st>>>(cp->nnodes, cp->brp, cp->bcol, f.slot_fine, fp->brp, fp->bcol,
+                                                      f.values, f.map, fp->bc, c.own_values);
+      break;
+   case 16:
+      mg_rap_kernel<16, W><<<grid, kMgThreads, 0, st>>>(cp->nnodes, cp->brp, cp->bcol, f.slot_fine, fp->brp, fp->bcol,
+                                                       f.values, f.map, fp->bc, c.own_values);
+      break;
+   default:
+      mg_rap_kernel<32, W><<<grid, kMgThreads, 0, st>>>(cp->nnodes, cp->brp, cp->bcol, f.slot_fine, fp->brp, fp->bcol,
+                                                       f.values, f.map, fp->bc, c.own_values);
+   }
 }
 
 extern "C" int femb200_mg_galerkin(femb200_mg *mg, const double *d_fine_values, int level, void *stream)
@@ -546,39 +703,41 @@ extern "C" int femb200_mg_galerkin(femb200_mg *mg, const double *d_fine_values, 
    FEMB_CHECK(mg, "mg_galerkin: null handle");
    const int L = (int)mg->lev.size() - 1;
    FEMB_CHECK(level >= 0 && level < L, "mg_galerkin: level %d outside [0, %d)", level, L);
-   if (level == 0)
+   const bool elem = level == 0 && mg->lev[0].pa;  // matrix-free level 0: element Galerkin step
+   if (elem)
+      FEMB_CHECK(!d_fine_values, "mg_galerkin: the fine level is matrix-free: pass no fine values (NULL)");
+   else if (level == 0)
    {
       FEMB_CHECK(d_fine_values, "mg_galerkin: null fine values");
       mg->lev[0].values = d_fine_values;
    }
-   FEMB_CHECK(mg->lev[level].values, "mg_galerkin: level %d has no values yet", level);
+   FEMB_CHECK(elem || mg->lev[level].values, "mg_galerkin: level %d has no values yet", level);
    const MgLevel &f = mg->lev[level];
    MgLevel &c = mg->lev[level + 1];
-   const femb200_plan *fp = f.plan, *cp = c.plan;
    cudaStream_t st = as_stream(stream);
-   const unsigned grid = (unsigned)cdiv(cp->nnodes * f.group, kMgThreads);
-   switch (f.group)
+   if (elem)
    {
-   case 8:
-      mg_rap_kernel<8><<<grid, kMgThreads, 0, st>>>(cp->nnodes, cp->brp, cp->bcol, f.slot_fine, fp->brp, fp->bcol, f.values,
-                                                   f.map, fp->bc, c.own_values);
-      break;
-   case 16:
-      mg_rap_kernel<16><<<grid, kMgThreads, 0, st>>>(cp->nnodes, cp->brp, cp->bcol, f.slot_fine, fp->brp, fp->bcol,
-                                                    f.values, f.map, fp->bc, c.own_values);
-      break;
-   default:
-      mg_rap_kernel<32><<<grid, kMgThreads, 0, st>>>(cp->nnodes, cp->brp, cp->bcol, f.slot_fine, fp->brp, fp->bcol,
-                                                    f.values, f.map, fp->bc, c.own_values);
+      if (int rc = pa_element_galerkin(f.pa, c.plan, c.own_values, st)) return rc;
    }
-   FEMB_LAUNCH_CHECK();
+   else
+   {
+      if (mg->width == 2)
+         mg_rap_launch<2>(f, c, st);
+      else
+         mg_rap_launch<4>(f, c, st);
+      FEMB_LAUNCH_CHECK();
+   }
    mg->have_inverse = false;
-   return femb200_apply_dirichlet(cp, c.own_values, 1.0, stream);
+   return femb200_apply_dirichlet(c.plan, c.own_values, 1.0, stream);
 }
 
 extern "C" int femb200_mg_setup(femb200_mg *mg, const double *d_fine_values, void *stream)
 {
-   FEMB_CHECK(mg && d_fine_values, "mg_setup: bad argument");
+   FEMB_CHECK(mg, "mg_setup: bad argument");
+   if (mg->lev[0].pa)
+      FEMB_CHECK(!d_fine_values, "mg_setup: the fine level is matrix-free: pass no fine values (NULL)");
+   else
+      FEMB_CHECK(d_fine_values, "mg_setup: bad argument");
    cudaStream_t st = as_stream(stream);
    const int L = (int)mg->lev.size() - 1;
    for (int l = 0; l < L; ++l)
@@ -587,7 +746,12 @@ extern "C" int femb200_mg_setup(femb200_mg *mg, const double *d_fine_values, voi
    for (int l = 0; l < L; ++l)
    {
       MgLevel &v = mg->lev[l];
-      if (int rc = femb200_extract_diagonal(v.plan, v.values, v.dinv, stream)) return rc;
+      if (v.pa)
+      {  // carries diag on the constrained dofs (femb200_pa_set_dirichlet), as the assembled diagonal does
+         if (int rc = femb200_pa_diagonal(v.pa, v.dinv, stream)) return rc;
+      }
+      else if (int rc = femb200_extract_diagonal(v.plan, v.values, v.dinv, stream))
+         return rc;
       if (int rc = femb200_jacobi_setup(v.n, v.dinv, v.dinv, stream)) return rc;
       // the fused-reduction scratch is taken right before every reducing kernel: an SpMV launch in between may grow
       // (reallocate) the scratch of the stream
@@ -600,7 +764,7 @@ extern "C" int femb200_mg_setup(femb200_mg *mg, const double *d_fine_values, voi
       FEMB_LAUNCH_CHECK();
       for (int it = 0; it < kPowerIters; ++it)
       {
-         if (int rc = femb200_spmv(v.plan, v.values, v.d, v.t, stream)) return rc;
+         if (int rc = mg_apply(mg, l, v.d, v.t, st)) return rc;
          if (int rc = reduce_scratch(grid, st, &red)) return rc;
          mg_scale_dot_kernel<<<grid, kMgThreads, 0, st>>>(v.n, v.dinv, v.t, v.r, red, mg->scal + l);
          FEMB_LAUNCH_CHECK();
@@ -670,9 +834,15 @@ extern "C" int femb200_mg_restrict(const femb200_mg *mg, int level, const double
    const int L = (int)mg->lev.size() - 1;
    FEMB_CHECK(level >= 0 && level < L, "mg_restrict: level %d outside [0, %d)", level, L);
    const MgLevel &f = mg->lev[level], &c = mg->lev[level + 1];
-   mg_restrict_kernel<<<(unsigned)cdiv(c.nnodes, kMgThreads), kMgThreads, 0, as_stream(stream)>>>(
-       c.nnodes, c.plan->brp, c.plan->bcol, f.slot_fine, f.plan->bc, c.plan->bc, reinterpret_cast<const double2 *>(d_b),
-       reinterpret_cast<const double2 *>(d_t), reinterpret_cast<double2 *>(d_bc));
+   const unsigned grid = (unsigned)cdiv(c.nnodes, kMgThreads);
+   const auto b = reinterpret_cast<const double2 *>(d_b), t = reinterpret_cast<const double2 *>(d_t);
+   const auto out = reinterpret_cast<double2 *>(d_bc);
+   if (mg->width == 2)
+      mg_restrict_kernel<2><<<grid, kMgThreads, 0, as_stream(stream)>>>(c.nnodes, c.plan->brp, f.slot_fine, f.map,
+                                                                         level_bc(f), level_bc(c), b, t, out);
+   else
+      mg_restrict_kernel<4><<<grid, kMgThreads, 0, as_stream(stream)>>>(c.nnodes, c.plan->brp, f.slot_fine, f.map,
+                                                                         level_bc(f), level_bc(c), b, t, out);
    FEMB_LAUNCH_CHECK();
    return 0;
 }
@@ -683,8 +853,13 @@ extern "C" int femb200_mg_prolong(const femb200_mg *mg, int level, const double 
    const int L = (int)mg->lev.size() - 1;
    FEMB_CHECK(level >= 0 && level < L, "mg_prolong: level %d outside [0, %d)", level, L);
    const MgLevel &f = mg->lev[level], &c = mg->lev[level + 1];
-   mg_prolong_kernel<<<(unsigned)cdiv(f.nnodes, kMgThreads), kMgThreads, 0, as_stream(stream)>>>(
-       f.nnodes, f.map, f.plan->bc, c.plan->bc, d_xc, d_x);
+   const unsigned grid = (unsigned)cdiv(f.nnodes, kMgThreads);
+   if (mg->width == 2)
+      mg_prolong_kernel<2><<<grid, kMgThreads, 0, as_stream(stream)>>>(f.nnodes, f.map, level_bc(f), level_bc(c), d_xc,
+                                                                        d_x);
+   else
+      mg_prolong_kernel<4><<<grid, kMgThreads, 0, as_stream(stream)>>>(f.nnodes, f.map, level_bc(f), level_bc(c), d_xc,
+                                                                        d_x);
    FEMB_LAUNCH_CHECK();
    return 0;
 }
@@ -735,7 +910,7 @@ int mg_smooth(const femb200_mg *mg, int l, const double *b, double *x, bool xzer
    const unsigned grid = mg_grid(n2);
    if (!xzero)
    {
-      if (int rc = femb200_spmv(v.plan, v.values, x, v.t, st)) return rc;
+      if (int rc = mg_apply(mg, l, x, v.t, st)) return rc;
       MG_MARK(tm, l, MG_T_SPMV);
    }
    mg_cheb_first_kernel<<<grid, kMgThreads, 0, st>>>(
@@ -746,7 +921,7 @@ int mg_smooth(const femb200_mg *mg, int l, const double *b, double *x, bool xzer
    MG_MARK(tm, l, MG_T_CHEB);
    for (int s = 1; s < mg->degree; ++s)
    {
-      if (int rc = femb200_spmv(v.plan, v.values, v.d, v.t, st)) return rc;
+      if (int rc = mg_apply(mg, l, v.d, v.t, st)) return rc;
       MG_MARK(tm, l, MG_T_SPMV);
       mg_cheb_step_kernel<<<grid, kMgThreads, 0, st>>>(n2, reinterpret_cast<const double2 *>(v.t),
                                                        reinterpret_cast<const double2 *>(v.dinv), reinterpret_cast<double2 *>(v.r),
@@ -771,7 +946,7 @@ int mg_vcycle_level(const femb200_mg *mg, int l, const double *b, double *x, cud
    }
    const MgLevel &c = mg->lev[l + 1];
    if (int rc = mg_smooth(mg, l, b, x, true, st, tm)) return rc;
-   if (int rc = femb200_spmv(v.plan, v.values, x, v.t, st)) return rc;
+   if (int rc = mg_apply(mg, l, x, v.t, st)) return rc;
    MG_MARK(tm, l, MG_T_SPMV);
    if (int rc = femb200_mg_restrict(mg, l, b, v.t, c.b, st)) return rc;
    MG_MARK(tm, l, MG_T_RESTRICT);
@@ -830,10 +1005,13 @@ extern "C" int femb200_pcg_mg(femb200_mg *mg, const double *d_b, double *d_x, do
    const int64_t n = f.n, n2 = n / 2;
    double *r = d_work, *d = d_work + n, *z = d_work + 2 * n, *Ad = d_work + 3 * n, *scal = d_work + 4 * n;
    RowRange rr{0, 0, {0, 0}};
-   if (int rc = plan_row_range(f.plan, 0, f.nnodes, &rr)) return rc;
+   if (f.plan)
+      if (int rc = plan_row_range(f.plan, 0, f.nnodes, &rr)) return rc;
    const unsigned grid = mg_grid(n2);
-   auto apply = [&]() -> int {
-      if (int rc = spmv_launch(f.plan, rr, f.values, d, Ad, scal + SC_FLAG, scal + SC_RED_DEN, false, st)) return rc;
+   auto apply = [&]() -> int {  // Ad = A d with the fused <d, A d> (SpMV or matrix-free apply)
+      if (int rc = f.pa ? pa_apply_launch(f.pa, d, Ad, scal + SC_FLAG, scal + SC_RED_DEN, st, false)
+                        : spmv_launch(f.plan, rr, f.values, d, Ad, scal + SC_FLAG, scal + SC_RED_DEN, false, st))
+         return rc;
       return femb200_cg_scalar_step(scal, 1, st);
    };
    auto precond_dot = [&](int red_slot) -> int {

@@ -205,7 +205,7 @@ __device__ __forceinline__ int rotated_local(int t, int a)
 }
 
 // --- slot map: position of every local dof b of visit (I, e, a) in block row I ---
-__global__ void k_fill_slots(int64_t nnodes, int nd, const int32_t *__restrict__ dofmap,
+__global__ void k_fill_slots(int64_t nnodes, int nd, bool rotated, const int32_t *__restrict__ dofmap,
                              const int32_t *__restrict__ nptr, const uint32_t *__restrict__ vis,
                              const int64_t *__restrict__ brp, const int32_t *__restrict__ bcol,
                              VisitRec *__restrict__ vrec)
@@ -226,7 +226,7 @@ __global__ void k_fill_slots(int64_t nnodes, int nd, const int32_t *__restrict__
       for (int b = 0; b < 8; ++b) r.slot[b] = 0;
       for (int t = 0; t < nd; ++t)
       {  // stored position t: triangles keep the columns in ROTATED order (plan.cuh), quads in natural order
-         const int b = nd <= 6 ? rotated_local(t, (int)r.a) : t;
+         const int b = rotated ? rotated_local(t, (int)r.a) : t;
          const int32_t J = dofmap[(int64_t)r.e * nd + b];
          int lo = 0, hi = deg;
          while (lo < hi)
@@ -607,7 +607,7 @@ extern "C" int femb200_plan_create(int etype, int64_t nnodes, int64_t ncells, co
 {
    FEMB_CHECK(out != nullptr, "plan_create: out is null");
    *out = nullptr;
-   FEMB_CHECK(etype >= FEMB200_P1 && etype <= FEMB200_Q2, "plan_create: unknown element family %d", etype);
+   FEMB_CHECK(etype >= FEMB200_P1 && etype <= FEMB200_Q1, "plan_create: unknown element family %d", etype);
    FEMB_CHECK(nnodes > 0 && ncells > 0, "plan_create: empty mesh (nnodes=%lld ncells=%lld)", (long long)nnodes,
               (long long)ncells);
    FEMB_CHECK(d_dofmap && d_xdofmap, "plan_create: null dofmap");
@@ -658,7 +658,8 @@ extern "C" int femb200_plan_create(int etype, int64_t nnodes, int64_t ncells, co
    cudaMemsetAsync(cnt, 0, sizeof(int32_t) * ((size_t)nnodes + 1), st);
    k_fill_visits<<<(unsigned)cdiv(nvis, T), T, 0, st>>>(nvis, nd, d_dofmap, p->nptr, cnt, tmpvis);
    k_sort_visits<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, p->nptr, tmpvis);
-   if (etype != FEMB200_Q2) k_order_visits<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, nd, d_dofmap, p->nptr, tmpvis);
+   const bool tri = elem_is_triangle(etype);  // quadrilaterals (Q2, Q1): no fan order, natural columns, no fast records
+   if (tri) k_order_visits<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, nd, d_dofmap, p->nptr, tmpvis);
 
    // 2. block degrees -> brp -> bcol
    if (dev_alloc(&deg, (size_t)nnodes + 1, &scratch) || dev_alloc(&p->brp, (size_t)nnodes + 4, &p->bytes))
@@ -696,7 +697,7 @@ extern "C" int femb200_plan_create(int etype, int64_t nnodes, int64_t ncells, co
    }
 
    // 3. slot map + staging-tile sizes
-   k_fill_slots<<<(unsigned)cdiv(nnodes, 128), 128, 0, st>>>(nnodes, nd, d_dofmap, p->nptr, tmpvis, p->brp, p->bcol,
+   k_fill_slots<<<(unsigned)cdiv(nnodes, 128), 128, 0, st>>>(nnodes, nd, tri, d_dofmap, p->nptr, tmpvis, p->brp, p->bcol,
                                                               p->vrec);
    {  // tile-sorted storage order (the slot map above was written node by node into a scratch copy)
       const int64_t ntiles = cdiv(nnodes, kAsmR);
@@ -723,7 +724,7 @@ extern "C" int femb200_plan_create(int etype, int64_t nnodes, int64_t ncells, co
 
    // fast-path records: triangles whose kAsmR-row staging image is addressable with 15-bit byte offsets
    // and whose nodes belong to fewer than 16 cells
-   if (etype != FEMB200_Q2 && 32 * ((int64_t)p->tile_max_blocks[1] + 8) < 32768 && p->max_deg < 128)
+   if (tri && 32 * ((int64_t)p->tile_max_blocks[1] + 8) < 32768 && p->max_deg < 128)
    {
       const int64_t ntiles = cdiv(nnodes, kAsmR);
       if (dev_alloc(&p->thdr, (size_t)ntiles, &p->bytes)) return fail(1);

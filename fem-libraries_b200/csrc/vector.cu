@@ -384,6 +384,7 @@ extern "C" int femb200_assemble_vector(const femb200_plan *p, const double *d_x,
                                        double *d_b, void *stream)
 {
    FEMB_CHECK(p && d_x && d_E && d_u && d_b, "assemble_vector: null argument");
+   FEMB_REFUSE_Q1(p->etype, "assemble_vector");
    FEMB_CHECK(x_stride == 2 || x_stride == 3, "assemble_vector: x_stride must be 2 or 3, got %d", x_stride);
    VecArgs A;
    A.nnodes = p->nnodes, A.nptr = p->nptr, A.vrec = p->vrec, A.perm = p->perm, A.voff = p->voff;
@@ -423,6 +424,7 @@ extern "C" int femb200_apply_lifting(const femb200_plan *p, const double *d_valu
                                      const double *d_u, double scale, double *d_b, double *d_work, void *stream)
 {
    FEMB_CHECK(p && d_values_nobc && d_g && d_u && d_b, "apply_lifting: null argument");
+   FEMB_REFUSE_Q1(p->etype, "apply_lifting");
    FEMB_CHECK(p->bc != nullptr, "apply_lifting: no Dirichlet dofs set on the plan");
    (void)d_work;  // scratch of the former SpMV form; kept in the signature
    if (p->nlift == 0) return 0;

@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("FEMB200_LIB") or os.path.join(os.path.dirname(_HERE), "lib", "libfemb200.so")
 
-P1, P2, Q2 = 0, 1, 2
+P1, P2, Q2, Q1 = 0, 1, 2, 3
 ROWMAJOR_INTERLEAVED, COLMAJOR_BYNODES = 0, 1
 TANGENT_CLOSED, TANGENT_AD = 0, 1
 OP_CSR, OP_PA = 0, 1
@@ -87,6 +87,7 @@ SIGNATURES = {
     "femb200_smooth_damage": [vp, vp, vp, i32, f64, vp],
     "femb200_cell_strain_stress": [i32, i64, vp, vp, vp, i32, vp, f64, vp, vp, vp, vp, vp],
     "femb200_mg_create": [vp, i32, vp, vp, vp, i32, f64, vp, C.POINTER(vp)],
+    "femb200_mg_create_op": [i32, vp, i32, vp, vp, i32, vp, i32, f64, vp, C.POINTER(vp)],
     "femb200_mg_sizes": [vp, C.POINTER(C.c_int), vp, vp, vp, C.POINTER(i64)],
     "femb200_mg_galerkin": [vp, vp, i32, vp],
     "femb200_mg_setup": [vp, vp, vp],

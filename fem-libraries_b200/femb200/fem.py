@@ -103,6 +103,8 @@ class ElasticityForm:
     (manual.py:19) and current iterate u (manual.py:30)."""
 
     def __init__(self, mesh: Mesh, E, nu: float = 0.3, d=None, u=None, variant: int = capi.TANGENT_CLOSED):
+        if mesh.etype == capi.Q1:
+            raise ValueError("ElasticityForm: Q1 meshes are pattern only (coarse multigrid levels); there is no Q1 element")
         self.mesh = mesh
         self.etype, self.nnodes, self.ncells = mesh.etype, mesh.nnodes, mesh.ncells
         self.nd, self.nv = mesh.nd, mesh.nv
@@ -582,10 +584,12 @@ class PAOperator:
         self._pa = C.c_void_p()
         self._bcs, self._diag = bcs, float(diag)
         self.bc_dev = None
+        self.generation = 0   # counts the AssemblePA calls: each one replaces the device operator behind `handle`
         self.AssemblePA()
 
     def AssemblePA(self):
         f = self.form
+        self.generation += 1
         if self._pa.value:
             capi.lib().femb200_pa_destroy(self._pa)
             self._pa = C.c_void_p()
@@ -631,26 +635,51 @@ class PAOperator:
 
 
 class MultigridPreconditioner:
-    """Geometric multigrid V-cycle for an assembled operator `A` (a Matrix with its Dirichlet conditions set) on a
-    nested MeshHierarchy whose finest mesh is A's mesh (mesh.lattice_hierarchy, mesh.refine_uniform_hierarchy).
+    """Geometric multigrid V-cycle for an operator `A` with its Dirichlet conditions set -- an assembled Matrix (P1, P2,
+    Q2) or a matrix-free PAOperator (P2, Q2) -- on a nested MeshHierarchy whose finest mesh is A's mesh
+    (mesh.lattice_hierarchy, mesh.quad_lattice_hierarchy, mesh.refine_uniform_hierarchy).
 
     Levels: A itself, then the Galerkin operators P^T A P of the coarser meshes, computed on the device by
     femb200_mg_setup; the hierarchy is cut at the first level with at most `coarse_max` dofs, whose dense inverse
-    (torch.linalg on the device) is the coarse solve.  Smoother: Chebyshev of `degree` on D^-1 A over
-    [lo_frac lambda, lambda], the same before and after the coarse correction, so the V-cycle is symmetric positive
-    definite.  Call setup() after every reassembly of A.values (the V-cycle reads A.values in place)."""
+    (torch.linalg on the device) is the coarse solve.  For a PAOperator the first step must be a p-coarsening (P2 -> P1,
+    Q2 -> Q1 on the same cells): its Galerkin operator is summed from the operator's per-cell data, the fine matrix is
+    never assembled.  Smoother: Chebyshev of `degree` on D^-1 A over [lo_frac lambda, lambda], the same before and after
+    the coarse correction, so the V-cycle is symmetric positive definite.  Call setup() after every reassembly of
+    A.values (the V-cycle reads A.values in place) or of the PAOperator: PAOperator.AssemblePA replaces the device
+    operator, so setup() then rebuilds the device handle on the new one, and apply() / solve() refuse to run until it has."""
 
-    def __init__(self, A: Matrix, hierarchy, degree: int = 2, coarse_max: int = 4096, lo_frac: float = 0.25):
-        from .mesh import P1
+    def __init__(self, A, hierarchy, degree: int = 2, coarse_max: int = 4096, lo_frac: float = 0.25):
+        from .mesh import P1, P2, Q1, Q2, ELEM_NAME
         _require_cuda()
+        if not isinstance(A, (Matrix, PAOperator)):
+            raise ValueError("the multigrid preconditioner needs a Matrix or a PAOperator")
+        self.matrix_free = isinstance(A, PAOperator)
         fine = hierarchy.meshes[-1]
-        if fine.ndofs != A.ndofs or fine.etype != A.form.etype:
+        mine = A.form.mesh
+        same = fine is mine or (fine.ndofs == A.ndofs and fine.etype == A.form.etype and fine.ncells == mine.ncells and
+                                np.array_equal(fine.dofmap, mine.dofmap) and np.array_equal(fine.x, mine.x))
+        if not same:
             raise ValueError(f"the finest mesh of the hierarchy ({fine.ndofs} dofs) is not the mesh of the operator "
                              f"({A.ndofs} dofs)")
         nlev = len(hierarchy.meshes)
         sizes = [m.ndofs for m in hierarchy.meshes]
         if nlev < 2:
             raise ValueError("the hierarchy has no mesh coarser than the fine one")
+        widths = {int(np.asarray(t).shape[1]) for t in hierarchy.maps}
+        if len(widths) != 1 or not widths <= {2, 4}:
+            raise ValueError(f"the transfer maps must all have width 2 or all width 4, got widths {sorted(widths)}")
+        self.width = widths.pop()
+        coarse_type = P1 if self.width == 2 else Q1
+        for m in hierarchy.meshes[:-1]:
+            if m.etype != coarse_type:
+                raise ValueError(f"coarse levels must be {ELEM_NAME[coarse_type]} for transfer maps of width "
+                                 f"{self.width}, got {ELEM_NAME.get(m.etype, m.etype)}")
+        if self.matrix_free:
+            first = hierarchy.meshes[-2]
+            want = {P2: P1, Q2: Q1}.get(fine.etype)
+            if want is None or first.etype != want or first.ncells != fine.ncells:
+                raise ValueError("a matrix-free (PAOperator) fine level needs a P2 or Q2 mesh whose first coarsening is a "
+                                 "p-coarsening (P2 -> P1 or Q2 -> Q1 on the same cells)")
         keep = next((k for k in range(nlev - 2, -1, -1) if sizes[k] <= coarse_max), None)
         if keep is None:
             raise ValueError(f"the coarsest mesh of the hierarchy has {sizes[0]} dofs, more than coarse_max = {coarse_max}")
@@ -665,23 +694,46 @@ class MultigridPreconditioner:
         self._plans = []
         for k in range(self.nlevels - 1, -1, -1):  # coarse levels 1 .. L
             m = meshes[k]
-            if m.etype != P1:
-                raise ValueError("coarse levels must be P1")
             dm = to_device(m.dofmap, np.int32)
             plan = C.c_void_p()
-            capi.call("femb200_plan_create", capi.P1, m.nnodes, m.ncells, _p(dm), _p(dm), _stream(), C.byref(plan))
+            capi.call("femb200_plan_create", m.etype, m.nnodes, m.ncells, _p(dm), _p(dm), _stream(), C.byref(plan))
             self._plans.append(plan)
             self._keep.append(dm)
         dmaps = [to_device(maps[k], np.int32) for k in range(self.nlevels - 1, -1, -1)]
         dbcs = [to_device(markers[k], np.uint8) for k in range(self.nlevels - 1, -1, -1)]
         self._keep += dmaps + dbcs
-        arr = lambda ts: (C.c_void_p * len(ts))(*[t.value if isinstance(t, C.c_void_p) else t.data_ptr() for t in ts])
+        self._dmaps, self._dbcs, self._lo_frac = dmaps, dbcs, float(lo_frac)
         self._handle = C.c_void_p()
-        capi.call("femb200_mg_create", A.plan, self.nlevels, arr(self._plans), arr(dmaps), arr(dbcs), self.degree,
-                  float(lo_frac), _stream(), C.byref(self._handle))
+        self._create()
         self.level_meshes = list(reversed(meshes))  # fine first
         self._work = None
         self.ready = False
+
+    def _create(self):
+        """The device handle on the operator as it is now (it borrows the operator, the plans, maps and markers)."""
+        arr = lambda ts: (C.c_void_p * len(ts))(*[t.value if isinstance(t, C.c_void_p) else t.data_ptr() for t in ts])
+        kind, op = (capi.OP_PA, self.A.handle) if self.matrix_free else (capi.OP_CSR, self.A.plan)
+        capi.call("femb200_mg_create_op", kind, op, self.nlevels, arr(self._plans), arr(self._dmaps), self.width,
+                  arr(self._dbcs), self.degree, self._lo_frac, _stream(), C.byref(self._handle))
+        self._generation = getattr(self.A, "generation", 0)
+
+    def _sync_operator(self):
+        """After PAOperator.AssemblePA the handle points at a freed operator: build it again on the new one."""
+        if self.matrix_free and self.A.generation != self._generation:
+            self.ready = False
+            capi.lib().femb200_mg_destroy(self._handle)
+            self._handle = C.c_void_p()
+            self._create()
+
+    def _check_ready(self, what: str):
+        if self.matrix_free and self.A.generation != self._generation:
+            raise RuntimeError(f"MultigridPreconditioner.{what}: the PAOperator was reassembled (AssemblePA); "
+                               "call setup() first")
+        if not self.ready:
+            raise RuntimeError(f"MultigridPreconditioner.{what}: call setup() first")
+
+    def _fine_values(self):
+        return None if self.matrix_free else _p(self.A.values)
 
     def close(self):
         if getattr(self, "_handle", None) is not None and self._handle.value:
@@ -716,12 +768,15 @@ class MultigridPreconditioner:
         return self.sizes()[2]
 
     def galerkin(self, level: int):
-        """Recompute A_{level+1} = P^T A_level P alone (timing and tests; setup() runs every level)."""
-        capi.call("femb200_mg_galerkin", self._handle, _p(self.A.values), int(level), _stream())
+        """Recompute A_{level+1} = P^T A_level P alone (timing and tests; setup() runs every level).  Level 0 of a
+        matrix-free operator is the element Galerkin step."""
+        self._sync_operator()
+        capi.call("femb200_mg_galerkin", self._handle, self._fine_values() if level == 0 else None, int(level), _stream())
 
     def setup(self):
         """Numeric phase: Galerkin cascade, smoother set-up (D^-1, lambda) and the coarse inverse."""
-        capi.call("femb200_mg_setup", self._handle, _p(self.A.values), _stream())
+        self._sync_operator()
+        capi.call("femb200_mg_setup", self._handle, self._fine_values(), _stream())
         self.set_coarse_inverse()
 
     def set_coarse_inverse(self):
@@ -738,7 +793,7 @@ class MultigridPreconditioner:
         return out
 
     def level_values(self, level: int) -> torch.Tensor:
-        """CSR values of level 1..L in the pattern of that level's P1 plan (level_csr)."""
+        """CSR values of level 1..L in the pattern of that level's P1 / Q1 plan (level_csr)."""
         out = torch.empty(self.sizes()[1][level], dtype=torch.float64, device="cuda")
         capi.call("femb200_mg_level_values", self._handle, int(level), _p(out), _stream())
         return out
@@ -755,18 +810,19 @@ class MultigridPreconditioner:
     def restrict(self, level: int, b: torch.Tensor, t: torch.Tensor | None = None) -> torch.Tensor:
         """P^T (b - t) from `level` to level + 1 (t = A x, or None for x = 0)."""
         out = torch.empty(self.sizes()[0][level + 1], dtype=torch.float64, device="cuda")
+        self._sync_operator()
         capi.call("femb200_mg_restrict", self._handle, int(level), _p(b), _p(t), _p(out), _stream())
         return out
 
     def prolong(self, level: int, xc: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
         """x += P xc from level + 1 to `level` (in place)."""
+        self._sync_operator()
         capi.call("femb200_mg_prolong", self._handle, int(level), _p(xc), _p(x), _stream())
         return x
 
     def apply(self, r: torch.Tensor, z: torch.Tensor | None = None) -> torch.Tensor:
         """z = B r: one V-cycle."""
-        if not self.ready:
-            raise RuntimeError("MultigridPreconditioner.apply: call setup() first")
+        self._check_ready("apply")
         if z is None:
             z = torch.empty_like(r)
         elif z.data_ptr() == r.data_ptr():
@@ -779,8 +835,7 @@ class MultigridPreconditioner:
     def apply_timed(self, r: torch.Tensor, z: torch.Tensor) -> np.ndarray:
         """One V-cycle with a CUDA event after every launch: (levels, 5) milliseconds per level of its SpMVs,
         Chebyshev vector passes, restriction, prolongation and coarse GEMV (femb200_mg_vcycle_timed)."""
-        if not self.ready:
-            raise RuntimeError("MultigridPreconditioner.apply_timed: call setup() first")
+        self._check_ready("apply_timed")
         if z.data_ptr() == r.data_ptr():
             raise ValueError("MultigridPreconditioner.apply_timed: z must not alias r")
         ms = np.zeros((self.nlevels + 1) * 5)
@@ -790,8 +845,7 @@ class MultigridPreconditioner:
     def solve(self, b: torch.Tensor, x: torch.Tensor, rel_tol: float = 1e-12, abs_tol: float = 0.0, max_iter: int = 2000,
               check_every: int = 1):
         """PCG on A with this preconditioner (femb200_pcg_mg): returns (iterations, final <B r, r>^1/2, converged)."""
-        if not self.ready:
-            raise RuntimeError("MultigridPreconditioner.solve: call setup() first")
+        self._check_ready("solve")
         n = self.A.ndofs
         if self._work is None or self._work.numel() < 4 * n + 64:
             self._work = torch.empty(4 * n + 64, dtype=torch.float64, device="cuda")
@@ -845,10 +899,11 @@ class CGSolver:
             self.dinv = None
             return
         if kind == "mg":
-            if not isinstance(self.op, Matrix):
-                raise ValueError("the multigrid preconditioner needs an assembled operator (Matrix)")
+            if not isinstance(self.op, (Matrix, PAOperator)):
+                raise ValueError("the multigrid preconditioner needs a Matrix or a PAOperator")
             if hierarchy is None:
-                raise ValueError('SetPreconditioner("mg") needs hierarchy= (mesh.lattice_hierarchy / refine_uniform_hierarchy)')
+                raise ValueError('SetPreconditioner("mg") needs hierarchy= (mesh.lattice_hierarchy / quad_lattice_hierarchy / '
+                                 'refine_uniform_hierarchy)')
             self.dinv = None
             self.mg = MultigridPreconditioner(self.op, hierarchy, **mg_options)
             self.mg.setup()

@@ -26,9 +26,10 @@ from dataclasses import dataclass, field
 import numpy as np
 
 P1, P2, Q2 = 0, 1, 2
-ELEM_ND = {P1: 3, P2: 6, Q2: 9}
-ELEM_NV = {P1: 3, P2: 3, Q2: 4}
-ELEM_NAME = {P1: "P1", P2: "P2", Q2: "Q2"}
+Q1 = 3          # pattern only (coarse levels of a quadrilateral multigrid hierarchy): no element kernel accepts it
+ELEM_ND = {P1: 3, P2: 6, Q2: 9, Q1: 4}
+ELEM_NV = {P1: 3, P2: 3, Q2: 4, Q1: 4}
+ELEM_NAME = {P1: "P1", P2: "P2", Q2: "Q2", Q1: "Q1"}
 
 
 @dataclass
@@ -308,10 +309,17 @@ def refine_uniform(mesh: Mesh, levels: int = 1) -> Mesh:
 @dataclass
 class MeshHierarchy:
     """Nested meshes for geometric multigrid, coarsest first: meshes[-1] is the finest (the mesh being solved on),
-    every other mesh is P1.  maps[k] ((meshes[k + 1].nnodes, 2) int32) is the transfer from meshes[k + 1] to
-    meshes[k]: per fine node a pair (a, b) of coarse node ids, a == b for a node that coincides with coarse node a
-    (weight 1), otherwise the midpoint of the coarse edge (a, b) (weight 1/2 on each); both components alike.
-    Indexing and len() go over the meshes."""
+    every other mesh is P1 (triangles) or Q1 (quadrilaterals).  maps[k] is the transfer from meshes[k + 1] to
+    meshes[k], one row of coarse node ids per fine node, both components alike:
+
+    * (nf, 2) int32 pairs (a, b): a == b for a node that coincides with coarse node a (weight 1), otherwise the
+      midpoint of the coarse edge (a, b) (weight 1/2 on each);
+    * (nf, 4) int32 rows: (a, a, a, a) a coincident node, (a, b, a, b) the midpoint of the coarse edge (a, b),
+      (v00, v10, v01, v11) the centre of a coarse quad; each distinct entry weighs 1 / (number of distinct entries).
+
+    Entry k and its partner (width - 1 - k) name the coarse pairs a fine node stands for (its node, its edge, the two
+    diagonals of its quad).  In both widths column 0 equals column 1 for a coincident node only.  Indexing and len()
+    go over the meshes."""
     meshes: list
     maps: list
 
@@ -379,6 +387,56 @@ def lattice_hierarchy(fine: Mesh) -> MeshHierarchy:
         c = structured_triangles(cx, cy, order=1)
         co = coincident_nodes(tmap, c.nnodes)
         c = Mesh(P1, np.ascontiguousarray(cur.x[co]), c.xdofmap, c.dofmap, cx, cy, dict(c.meta))
+        meshes.insert(0, c)
+        maps.insert(0, tmap)
+        cur, mfx, mfy = c, cx + 1, cy + 1
+    return MeshHierarchy(meshes, maps)
+
+
+def _quad_lattice_map(mxf: int, myf: int) -> np.ndarray:
+    """Width-4 map of the (mxf x myf)-node lattice halved: node (i, j) -> the coarse lattice nodes (i // 2 or
+    (i + 1) // 2, j // 2 or (j + 1) // 2): (a, a, a, a) for even (i, j), (a, b, a, b) for the midpoint of a horizontal
+    or vertical coarse edge, (v00, v10, v01, v11) for odd (i, j), the centre of a coarse quad."""
+    mxc = (mxf - 1) // 2 + 1
+    i, j = np.meshgrid(np.arange(mxf, dtype=np.int64), np.arange(myf, dtype=np.int64), indexing="xy")
+    i, j = i.ravel(), j.ravel()
+    c = lambda ii, jj: ii + mxc * jj
+    i0, i1, j0, j1 = i // 2, (i + 1) // 2, j // 2, (j + 1) // 2
+    m = np.stack([c(i0, j0), c(i1, j0), c(i0, j1), c(i1, j1)], axis=1)
+    vert = (i % 2 == 0) & (j % 2 == 1)          # (a, a, b, b) -> (a, b, a, b)
+    m[vert] = m[vert][:, [0, 2, 0, 2]]
+    return np.ascontiguousarray(m.astype(np.int32))
+
+
+def _quads_q1(nx: int, ny: int, x: np.ndarray) -> Mesh:
+    """Q1 mesh of nx x ny cells on the (nx + 1) x (ny + 1) vertex lattice, cells in the order of structured_quads_q2
+    (x fastest), local order (v00, v10, v01, v11)."""
+    mx = nx + 1
+    cx, cy = np.meshgrid(np.arange(nx, dtype=np.int64), np.arange(ny, dtype=np.int64), indexing="xy")
+    v00 = (cx + mx * cy).ravel()
+    dm = np.stack([v00, v00 + 1, v00 + mx, v00 + mx + 1], axis=1).astype(np.int32)
+    return Mesh(Q1, np.ascontiguousarray(x), dm, dm.copy(), nx, ny, {"kind": "structured-quad", "order": 1})
+
+
+def quad_lattice_hierarchy(fine: Mesh) -> MeshHierarchy:
+    """Hierarchy of a `structured_quads_q2` mesh (any nx x ny, jittered or not): Q2 -> Q1 on the same vertices and the
+    same cells (cell k of the Q1 mesh is cell k of the Q2 mesh; the Q2 node lattice maps like a halved lattice), then
+    the Q1 lattice halved while both cell counts are even.  Width-4 maps; coarse nodes take the coordinates of their
+    coincident fine nodes."""
+    if fine.meta.get("kind") != "structured-quad" or fine.etype != Q2:
+        raise ValueError("quad_lattice_hierarchy: needs a Q2 mesh of structured_quads_q2")
+    meshes, maps = [fine], []
+    cur, mfx, mfy = fine, 2 * fine.nx + 1, 2 * fine.ny + 1
+    while True:
+        if cur is fine:
+            cx, cy = fine.nx, fine.ny
+        elif cur.nx % 2 == 0 and cur.ny % 2 == 0:
+            cx, cy = cur.nx // 2, cur.ny // 2
+        else:
+            break
+        tmap = _quad_lattice_map(mfx, mfy)
+        co = coincident_nodes(tmap, (cx + 1) * (cy + 1))
+        c = _quads_q1(cx, cy, cur.x[co])
         meshes.insert(0, c)
         maps.insert(0, tmap)
         cur, mfx, mfy = c, cx + 1, cy + 1

@@ -40,6 +40,8 @@ extern "C" {
 #define FEMB200_P1 0 /* P1 triangle, 1-point rule  (the reference: M.cc:511-512, manual.py:10,97) */
 #define FEMB200_P2 1 /* P2 triangle, 3-point rule, basix dof order                                */
 #define FEMB200_Q2 2 /* Q2 quadrilateral, 3x3 Gauss, tensor dof order                              */
+#define FEMB200_Q1 3 /* Q1 quadrilateral, pattern only: coarse levels of the multigrid hierarchy;
+                        local order (v00, v10, v01, v11); no element kernel accepts it            */
 
 /* element-matrix layouts */
 #define FEMB200_ROWMAJOR_INTERLEAVED 0 /* ufcx tabulate_tensor: A[(2a+i)*n + 2b+k]              */
@@ -355,20 +357,37 @@ int femb200_cell_strain_stress(int etype, int64_t ncells, const int32_t *d_xdofm
                                const double *d_u, double *d_strain, double *d_stress, void *stream);
 
 /* ------------------------------------------------------------------------
- * Geometric multigrid preconditioner (assembled CSR operator, single GPU).
- * Levels 0 (the fine plan, Dirichlet applied through its marker) .. L (coarsest); level l + 1 is a P1 plan.
- * Transfer map of level l: int32 pair (a, b) of level-(l+1) node ids per level-l node: a == b a coincident
- * node (weight 1), else the midpoint of the coarse edge (a, b) (weight 1/2 each), both components alike.
- * P has zero rows for constrained fine dofs and zero columns for constrained coarse dofs (the plans' markers).
- *   mg_create       borrows the plans (they must outlive the handle); sets the coarse plans' Dirichlet markers
- *                   from d_coarse_bc[l] (uint8 per dof, NULL: none); validates that the maps are nested (every
- *                   midpoint on an edge of the coarse pattern, every coarse node and edge hit once);
+ * Geometric multigrid preconditioner (single GPU).
+ * Levels 0 (the fine operator, Dirichlet applied through its marker) .. L (coarsest).  Level 0 is an assembled
+ * plan (FEMB200_OP_CSR: P1, P2 or Q2) or a matrix-free operator (FEMB200_OP_PA: P2 or Q2); levels 1..L are P1
+ * plans (map width 2) or Q1 plans (map width 4).
+ * Transfer map of level l, per level-l node, `width` int32 level-(l+1) node ids:
+ *   width 2  (a, b): a == b a coincident node (weight 1), else the midpoint of the coarse edge (a, b) (1/2 each);
+ *   width 4  (a, a, a, a) a coincident node, (a, b, a, b) the midpoint of edge (a, b), (v00, v10, v01, v11) the
+ *            centre of a coarse quad; each distinct entry weighs 1 / (number of distinct entries).
+ * Entry k and its partner (width - 1 - k) name the coarse block slots a fine node stands for: its diagonal block,
+ * its edge, or the two diagonals of its quad.  Both components alike.  P has zero rows for constrained fine dofs
+ * and zero columns for constrained coarse dofs (the levels' markers).
+ *   mg_create_op    borrows the fine operator and the plans (they must outlive the handle); sets the coarse plans'
+ *                   Dirichlet markers from d_coarse_bc[l] (uint8 per dof, NULL: none); validates that the maps
+ *                   are nested (every pair in the coarse pattern, every coarse slot hit by exactly one fine node);
  *                   Chebyshev smoother of `degree` on D^-1 A over [lo_frac lambda, lambda].  Synchronises.
- *   mg_sizes        host: L, and per level 0..L dofs, nnz, lambda (1.1 x 15-step power iteration, after setup)
+ *                   OP_CSR: fine_op is the fine plan.  OP_PA: fine_op is a femb200_pa (its own Dirichlet marker
+ *                   and diagonal, read at every call); the first step must be a p-coarsening (P2 -> P1, Q2 -> Q1):
+ *                   the map row of every node of fine cell k names the vertices of coarse cell k the element
+ *                   interpolation weights it on (checked on the device).  Destroying the operator invalidates the
+ *                   handle: create a new one on the new operator.
+ *   mg_create       = mg_create_op(FEMB200_OP_CSR, fine, ..., width 2, ...)
+ *   mg_sizes        host: L, and per level 0..L dofs, nnz (0 for a matrix-free level 0), lambda (1.1 x 15-step
+ *                   power iteration, after setup), device bytes of the handle
  *   mg_galerkin     A_{level+1} = P^T A_level P (gather kernel, write-once) + unit Dirichlet diagonal;
- *                   level 0 reads d_fine_values (kept by the handle: it must stay valid)
+ *                   level 0 reads d_fine_values (kept by the handle: it must stay valid).  Matrix-free level 0:
+ *                   d_fine_values must be NULL; sum over the cells of P_e^T K_e P_e from the operator's own
+ *                   geometry and quadrature, gathered through the coarse plan's visit records (no fine matrix;
+ *                   a per-cell scratch of (2 nv)^2 doubles is allocated on `stream` for the call only)
  *   mg_setup        the numeric phase: every mg_galerkin, D^-1 and lambda per level.  Synchronises.  Re-run
- *                   after every reassembly of the fine values, then hand in a new coarse inverse.
+ *                   after every reassembly of the fine values, then hand in a new coarse inverse.  d_fine_values:
+ *                   NULL for a matrix-free level 0.
  *   mg_level_values copy of the CSR values of level 1..L (the pattern of that level's plan)
  *   mg_coarse_matrix / mg_set_coarse_inverse: dense row-major image of A_L (n_L^2 doubles), and its inverse
  *                   (copied into the handle; the V-cycle applies it with a GEMV kernel)
@@ -382,6 +401,9 @@ typedef struct femb200_mg femb200_mg;
 int femb200_mg_create(const femb200_plan *fine, int nlevels, femb200_plan *const *coarse_plans,
                       const int32_t *const *d_maps, const uint8_t *const *d_coarse_bc, int degree, double lo_frac,
                       void *stream, femb200_mg **out);
+int femb200_mg_create_op(int op_kind, const void *fine_op, int nlevels, femb200_plan *const *coarse_plans,
+                         const int32_t *const *d_maps, int map_width, const uint8_t *const *d_coarse_bc, int degree,
+                         double lo_frac, void *stream, femb200_mg **out);
 void femb200_mg_destroy(femb200_mg *mg);
 int femb200_mg_sizes(const femb200_mg *mg, int *nlevels, int64_t *ndofs, int64_t *nnz, double *lambda,
                      int64_t *device_bytes);
