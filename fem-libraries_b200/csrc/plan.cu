@@ -507,6 +507,100 @@ __global__ void k_cols16(int64_t nnodes, const int64_t *__restrict__ brp, const 
    }
 }
 
+// --- stencil dictionary of the SpMV (plan.cuh) --------------------------------------------
+// Distinct bcol16 lists: an open-addressing table of kStencilH 64-bit list hashes (0: empty slot) with the first row
+// that has each list.  flags[0] is set when there are more than kStencilK lists, a row has more than kStencilD blocks or
+// an id does not verify; the table is then dropped and the plan has no stencil path.
+constexpr int kStencilH = 1024;
+
+__device__ __forceinline__ uint64_t stencil_hash(const int16_t *__restrict__ c, int deg)
+{
+   uint64_t h = 0xcbf29ce484222325ull ^ (uint64_t)deg;
+   for (int s = 0; s < deg; ++s)
+   {
+      h = (h ^ (uint16_t)c[s]) * 0x100000001b3ull;
+      h ^= h >> 29;
+   }
+   return h ? h : 1;
+}
+
+__global__ void k_stencil_insert(int64_t nnodes, const int64_t *__restrict__ brp, const int16_t *__restrict__ bcol16,
+                                 unsigned long long *keys, int32_t *first, int32_t *count, int32_t *flags)
+{
+   const int64_t I = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+   if (I >= nnodes || *(volatile int32_t *)flags) return;  // once it has failed, the remaining rows need not hash
+   const int64_t b0 = brp[I];
+   const int deg = (int)(brp[I + 1] - b0);
+   if (deg > kStencilD)
+   {
+      atomicOr(flags, 1);
+      return;
+   }
+   const unsigned long long h = stencil_hash(bcol16 + b0, deg);
+   unsigned s = (unsigned)(h >> 40) & (kStencilH - 1);
+   for (int probe = 0; probe < kStencilH; ++probe, s = (s + 1) & (kStencilH - 1))
+   {
+      unsigned long long k = *(volatile unsigned long long *)&keys[s];  // plain read first: almost every row finds its list
+      if (k == 0)
+      {
+         k = atomicCAS(&keys[s], 0ull, h);
+         if (k == 0 && atomicAdd(count, 1) >= kStencilK) atomicOr(flags, 1);
+      }
+      if (k == 0 || k == h)
+      {
+         if (*(volatile int32_t *)&first[s] > (int32_t)I) atomicMin(&first[s], (int32_t)I);
+         return;
+      }
+   }
+   atomicOr(flags, 1);  // table full
+}
+
+// one CTA of kStencilH threads: stencil id = rank of the list's first row (order of first appearance); writes the ids
+// into the table and each list's offsets and degree into the dictionary
+__global__ void __launch_bounds__(kStencilH)
+k_stencil_ids(const int64_t *__restrict__ brp, const int16_t *__restrict__ bcol16, const unsigned long long *__restrict__ keys,
+              const int32_t *__restrict__ first, int32_t *__restrict__ ids, int16_t *__restrict__ off, uint8_t *__restrict__ sdeg)
+{
+   __shared__ int32_t s_first[kStencilH];
+   const int s = threadIdx.x;
+   const bool used = keys[s] != 0;
+   s_first[s] = used ? first[s] : INT32_MAX;
+   __syncthreads();
+   if (!used) return;
+   int id = 0;
+   for (int t = 0; t < kStencilH; ++t) id += s_first[t] < s_first[s];
+   ids[s] = id;
+   const int64_t b0 = brp[s_first[s]];
+   const int deg = (int)(brp[s_first[s] + 1] - b0);
+   sdeg[id] = (uint8_t)deg;
+   for (int t = 0; t < kStencilD; ++t) off[id * kStencilD + t] = t < deg ? bcol16[b0 + t] : (int16_t)0;
+}
+
+// sig[I] = id of row I's list, then the verification: the row's degree and every offset equal its dictionary entry
+__global__ void k_stencil_assign(int64_t nnodes, const int64_t *__restrict__ brp, const int16_t *__restrict__ bcol16,
+                                 const unsigned long long *__restrict__ keys, const int32_t *__restrict__ ids,
+                                 const int16_t *__restrict__ off, const uint8_t *__restrict__ sdeg, uint8_t *__restrict__ sig,
+                                 int32_t *__restrict__ flags)
+{
+   const int64_t I = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+   if (I >= nnodes) return;
+   const int64_t b0 = brp[I];
+   const int deg = (int)(brp[I + 1] - b0);
+   const unsigned long long h = stencil_hash(bcol16 + b0, deg);
+   unsigned s = (unsigned)(h >> 40) & (kStencilH - 1);
+   for (int probe = 0; probe < kStencilH && keys[s] != h; ++probe) s = (s + 1) & (kStencilH - 1);
+   if (keys[s] != h)
+   {
+      atomicOr(flags, 1);
+      return;
+   }
+   const int id = ids[s];
+   sig[I] = (uint8_t)id;
+   bool ok = sdeg[id] == deg;
+   for (int t = 0; t < deg && ok; ++t) ok = off[id * kStencilD + t] == bcol16[b0 + t];
+   if (!ok) atomicOr(flags, 1);
+}
+
 __global__ void k_scalar_csr(int64_t nnodes, const int64_t *__restrict__ brp, const int32_t *__restrict__ bcol,
                              int64_t *__restrict__ rowptr, int32_t *__restrict__ colidx)
 {
@@ -570,6 +664,58 @@ static int dev_alloc(T **p, size_t n, size_t *acc)
    return 0;
 }
 
+// Stencil ids of the node rows (plan.cuh), from bcol16.  Leaves p->sig null (the SpMV then reads bcol16) when the
+// pattern has more than kStencilK distinct lists, a row longer than kStencilD, or a row that does not verify.
+static int plan_stencils(femb200_plan *p, cudaStream_t st)
+{
+   const int64_t nnodes = p->nnodes;
+   unsigned char *scratch = nullptr;  // keys [H] u64 | first [H] | ids [H] | count | flags
+   const size_t sbytes = kStencilH * (8 + 4 + 4) + 16;
+   FEMB_CUDA(cudaMalloc(&scratch, sbytes));
+   auto *keys = reinterpret_cast<unsigned long long *>(scratch);
+   auto *first = reinterpret_cast<int32_t *>(scratch + 8 * kStencilH);
+   auto *ids = first + kStencilH, *count = ids + kStencilH, *flags = count + 1;
+   size_t bytes = 0;
+   int rc = 0;
+   int32_t h[2] = {0, 0};
+   const int T = 256;
+   if ((rc = dev_alloc(&p->sig, (size_t)nnodes, &bytes)) || (rc = dev_alloc(&p->stencil_off, kStencilK * kStencilD, &bytes)) ||
+       (rc = dev_alloc(&p->stencil_deg, kStencilK, &bytes)))
+      goto done;
+   cudaMemsetAsync(keys, 0, 8 * kStencilH, st);
+   cudaMemsetAsync(first, 0x7f, 4 * kStencilH, st);  // 0x7f7f7f7f: above every node id
+   cudaMemsetAsync(count, 0, 8, st);
+   k_stencil_insert<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, p->brp, p->bcol16, keys, first, count, flags);
+   if (cudaMemcpyAsync(h, count, sizeof(h), cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess)
+   {
+      rc = set_error("plan_create: stencil table failed: %s", cudaGetErrorString(cudaGetLastError()));
+      goto done;
+   }
+   if (!h[1])
+   {
+      k_stencil_ids<<<1, kStencilH, 0, st>>>(p->brp, p->bcol16, keys, first, ids, p->stencil_off, p->stencil_deg);
+      k_stencil_assign<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, p->brp, p->bcol16, keys, ids, p->stencil_off,
+                                                               p->stencil_deg, p->sig, flags);
+      if (cudaMemcpyAsync(h + 1, flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+          cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess)
+      {
+         rc = set_error("plan_create: stencil ids failed: %s", cudaGetErrorString(cudaGetLastError()));
+         goto done;
+      }
+   }
+done:
+   cudaFree(scratch);
+   if (rc || h[1])
+   {
+      cudaFree(p->sig), cudaFree(p->stencil_off), cudaFree(p->stencil_deg);
+      p->sig = nullptr, p->stencil_off = nullptr, p->stencil_deg = nullptr;
+      return rc;
+   }
+   p->nstencils = h[0];
+   p->bytes += bytes;
+   return 0;
+}
+
 }  // namespace femb
 
 using namespace femb;
@@ -587,6 +733,9 @@ extern "C" void femb200_plan_destroy(femb200_plan *p)
    cudaFree(p->brp);
    cudaFree(p->bcol);
    cudaFree(p->bcol16);
+   cudaFree(p->sig);
+   cudaFree(p->stencil_off);
+   cudaFree(p->stencil_deg);
    cudaFree(p->dslot);
    cudaFree(p->bc);
    cudaFree(p->bc_nodes);
@@ -695,6 +844,7 @@ extern "C" int femb200_plan_create(int etype, int64_t nnodes, int64_t ncells, co
       }
       cudaMemsetAsync(flags, 0, sizeof(int32_t) * 2, st);
    }
+   if (p->bcol16 && (rc = plan_stencils(p, st))) return fail(rc);
 
    // 3. slot map + staging-tile sizes
    k_fill_slots<<<(unsigned)cdiv(nnodes, 128), 128, 0, st>>>(nnodes, nd, tri, d_dofmap, p->nptr, tmpvis, p->brp, p->bcol,
@@ -964,7 +1114,8 @@ extern "C" int femb200_plan_set_option(femb200_plan *p, const char *key, int val
    }
    else if (!strcmp(key, "spmv_cols"))
    {
-      FEMB_CHECK(value == 0 || value == 1, "plan_set_option: spmv_cols must be 0 (auto: 16-bit relative indices) or 1 (32-bit)");
+      FEMB_CHECK(value >= 0 && value <= 2,
+                 "plan_set_option: spmv_cols must be 0 (auto: stencil ids, else 16-bit offsets), 1 (32-bit) or 2 (16-bit offsets)");
       p->opt_spmv_cols = value;
    }
    else if (!strcmp(key, "vector_path"))
@@ -1003,7 +1154,9 @@ extern "C" int femb200_plan_get_option(const femb200_plan *p, const char *key, i
    else if (!strcmp(key, "stream_out"))
       *value = p->opt_stream_out;
    else if (!strcmp(key, "spmv_col_bits"))
-      *value = (p->bcol16 && p->opt_spmv_cols != 1) ? 16 : 32;
+      *value = (p->sig && p->opt_spmv_cols == 0) ? 0 : (p->bcol16 && p->opt_spmv_cols != 1) ? 16 : 32;
+   else if (!strcmp(key, "spmv_stencils"))
+      *value = p->sig ? p->nstencils : 0;
    else if (!strcmp(key, "fast_records"))
       *value = p->frec ? 1 : 0;
    else

@@ -100,6 +100,10 @@ constexpr int kAsmLevels = 16; // visits per node supported by the tile-sorted l
 static_assert(kAsmLevels == kAsmLevelsFwd, "TileHdr::voff");
 static_assert(sizeof(TileHdr) == 64, "TileHdr must be 64 bytes");
 constexpr int kNumTileR = 6;
+// Stencil dictionary of the SpMV (spmv.cu): the distinct lists of column offsets J - I of the node rows, at most
+// kStencilK lists of at most kStencilD offsets (a lattice numbering has a handful: 16 for P2 triangles).
+constexpr int kStencilK = 64;
+constexpr int kStencilD = 32;
 __host__ __device__ constexpr int tile_r(int r) { return r == 0 ? 32 : r == 1 ? 64 : r == 2 ? 96 : r == 3 ? 128 : r == 4 ? 192 : 256; }
 
 }  // namespace femb
@@ -121,6 +125,11 @@ struct femb200_plan
    int64_t *brp = nullptr;                                // [nnodes+1]
    int32_t *bcol = nullptr;                               // [nnzb]
    int16_t *bcol16 = nullptr;                             // [nnzb] bcol[k] - (node of the row), or null when one does not fit
+   // stencil ids (null / 0 when the pattern has no dictionary): row I's bcol16 list is stencil_off[sig[I]][0, deg)
+   uint8_t *sig = nullptr;                                // [nnodes] stencil id of each node row
+   int16_t *stencil_off = nullptr;                        // [nstencils][kStencilD] offsets, in the plan's column order
+   uint8_t *stencil_deg = nullptr;                        // [nstencils] block degree of each stencil
+   int32_t nstencils = 0;
    uint8_t *dslot = nullptr;                              // [nnodes] slot of the diagonal block in its row (255: none)
    int32_t tile_max_blocks[femb::kNumTileR] = {0, 0, 0, 0, 0, 0};
    // Dirichlet
@@ -152,7 +161,7 @@ struct femb200_plan
    // fast records / oversized SpMV tiles can be forced, so that the tests cover them on any mesh.
    int opt_assembly_path = 0;    // 0 auto; 1 visit-record kernel; 2 per-quadrature-point kernel
    int opt_spmv_path = 0;        // 0 auto (bulk-copy staged, persistent); 1 direct kernel
-   int opt_spmv_cols = 0;        // 0 auto (16-bit relative column indices when the pattern allows); 1 32-bit indices
+   int opt_spmv_cols = 0;        // 0 auto (stencil ids, else 16-bit relative indices, else 32-bit); 1 32-bit; 2 16-bit
    int opt_vector_path = 0;      // residual vector: 0 two passes (per-cell r_e + gather); 1 single-pass gather
    int opt_prefetch_tiles = -1;  // record prefetch distance of the assembly kernel in tiles (-1: 8 x SM count)
    // largest 32- / 64-row SpMV tile (in node blocks) of the tiling that starts at row_lo, per row range

@@ -82,7 +82,7 @@ spmv_kernel(int64_t row_lo, int64_t nnodes, const int64_t *__restrict__ brp, con
 // ---------------------------------------------------------------------------
 // TMA-staged persistent variant (default).  The node rows [n0, n0 + R) of a tile
 // own one contiguous byte range of the value array, of bcol and of brp: a producer
-// warp streams those three ranges into shared memory with 1-D bulk copies
+// warp streams those ranges into shared memory with 1-D bulk copies
 // (cp.async.bulk -> UBLKCP) completing on an mbarrier, S stages deep, while eight
 // consumer warps (L lanes per node row pair) reduce the previous tiles out of shared memory; the only
 // per-thread global loads left are the gathers of x (L1/L2 hits: the lattice
@@ -94,24 +94,57 @@ constexpr int kTmaThreads = kTmaConsumers + 32;
 
 struct SpmvTile
 {
-   int vbytes, cbytes, pbytes;  // stage capacities: values, column indices, row pointers
+   int vbytes, cbytes, pbytes;  // stage capacities: values, column indices (or stencil ids), row pointers
 };
 
-// C16: the column indices are the plan's 16-bit offsets from the row's own node (bcol16: every |J - I| of the pattern fits,
-// which any numbering with locality gives: the lattice numbering of config 4 has |J - I| <= 2 (2 n + 1) + 2 = 23 172):
-// 34 instead of 36 bytes per node block, 5 % of the kernel's DRAM traffic.
-template <bool DOT, int R, int kTmaStages, int L, bool C16>
+// Column modes.  C32: the plan's bcol.  C16: its 16-bit offsets from the row's own node (bcol16: every |J - I| of the
+// pattern fits, which any numbering with locality gives: the lattice numbering of config 4 has |J - I| <= 2 (2 n + 1) + 2
+// = 23 172): 34 instead of 36 bytes per node block.  STENCIL: one byte per node row, the row's id in the plan's stencil
+// dictionary (the distinct bcol16 lists: 16 on a P2 lattice), which the CTA holds in shared memory: 32 bytes per node
+// block and one per node row, no column indices and no brp stage.  The producer warp reads a tile's ids two tiles
+// ahead, turns them into value offsets (warp scan over the dictionary degrees) one tile ahead, and stores one word per
+// row, (offset | id << 16), into the stage next to the values before it arrives on the stage's barrier: the consumers'
+// dependent chain stays as short as with brp, and no global read sits between a free stage and its value copy (with
+// the scan in the consumers the apply was 4 % slower than the 16-bit mode).  All three modes apply the same products in
+// the same order: y and <x, y> agree bit for bit.
+enum SpmvCols
+{
+   kC32 = 0,
+   kC16 = 1,
+   kStencil = 2
+};
+// shared-memory dictionary entry: kStencilD offsets, the degree, one pad entry (17 words: rows of different ids start in
+// different banks)
+constexpr int kDictStride = kStencilD + 2;
+
+struct SpmvStencils
+{
+   const uint8_t *sig;       // [nnodes]
+   const int16_t *off;       // [k][kStencilD]
+   const uint8_t *deg;       // [k]
+   int k;
+};
+
+template <bool DOT, int R, int kTmaStages, int L, int COLS>
 __global__ void __launch_bounds__(kTmaThreads)
 spmv_tma_kernel(int64_t row_lo, int64_t row_hi, const int64_t *__restrict__ brp, const void *__restrict__ bcol_any,
-                const double *__restrict__ values, const double *__restrict__ x, double *__restrict__ y,
+                SpmvStencils dict, const double *__restrict__ values, const double *__restrict__ x, double *__restrict__ y,
                 const double *__restrict__ flag, ReduceScratch red, double *__restrict__ out, SpmvTile cap, int ntiles,
                 bool accumulate)
 {
+   static_assert(COLS != kStencil || R == 64, "the stencil scan covers 64 rows (two per lane of the producer warp)");
    extern __shared__ __align__(128) unsigned char smem[];
    __shared__ uint64_t full[kTmaStages], empty[kTmaStages];
    if (flag && *flag != 0.) return;  // converged CG: become a no-op (uniform over the grid)
    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
    const int stage_bytes = cap.vbytes + cap.cbytes + cap.pbytes;
+   int16_t *sdict = reinterpret_cast<int16_t *>(smem + (size_t)kTmaStages * stage_bytes);
+   if constexpr (COLS == kStencil)  // the dictionary, once per CTA (published by the __syncthreads below)
+      for (int e = tid; e < dict.k * kDictStride; e += kTmaThreads)
+      {
+         const int k = e / kDictStride, t = e - k * kDictStride;
+         sdict[e] = t < kStencilD ? dict.off[k * kStencilD + t] : t == kStencilD ? (int16_t)dict.deg[k] : (int16_t)0;
+      }
    if (tid == 0)
    {
 #pragma unroll
@@ -128,7 +161,57 @@ spmv_tma_kernel(int64_t row_lo, int64_t row_hi, const int64_t *__restrict__ brp,
    double part = 0.;
    if (warp == kTmaConsumers / 32)
    {  // ---- producer warp: one lane issues the bulk copies ----
-      if (lane == 0)
+      if constexpr (COLS == kStencil)
+      {  // the whole warp; lane l resolves rows 2 l and 2 l + 1.  What a tile needs besides its stage is prepared ahead
+         // while the consumers still hold the stages: the global reads (first node block, ids) two tiles ahead, the
+         // value offsets (scan) one tile ahead, so the value copy leaves as soon as its stage is free
+         const int r = 2 * lane;
+         auto rows = [&](int it) { return (int)min((int64_t)R, row_hi - (row_lo + (int64_t)(first + it * stride) * R)); };
+         int64_t rb0 = 0, b0 = 0;      // raw reads of the tile after next; first node block of the next tile
+         int rid0 = 0, rid1 = 0;
+         uint32_t w0 = 0u, w1 = 0u, vb = 0u;  // the next tile's words and value bytes
+         auto load = [&](int it) {
+            const int64_t n0 = row_lo + (int64_t)(first + it * stride) * R;
+            const int nloc = rows(it);
+            rb0 = brp[n0];
+            rid0 = r < nloc ? dict.sig[n0 + r] : 0, rid1 = r + 1 < nloc ? dict.sig[n0 + r + 1] : 0;
+         };
+         auto scan = [&](int it) {
+            const int nloc = rows(it);
+            const int d0 = r < nloc ? sdict[rid0 * kDictStride + kStencilD] : 0;
+            const int d1 = r + 1 < nloc ? sdict[rid1 * kDictStride + kStencilD] : 0;
+            int incl = d0 + d1;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1)
+            {
+               const int v = __shfl_up_sync(0xffffffffu, incl, o);
+               if (lane >= o) incl += v;
+            }
+            const uint32_t e0 = (uint32_t)(incl - d0 - d1);
+            w0 = e0 | ((uint32_t)rid0 << 16), w1 = (e0 + d0) | ((uint32_t)rid1 << 16);
+            vb = 32u * (uint32_t)__shfl_sync(0xffffffffu, incl, 31);  // the tile's blocks = brp[n0 + nloc] - brp[n0]
+            b0 = rb0;
+         };
+         if (nmine > 0) load(0), scan(0);
+         if (nmine > 1) load(1);
+         for (int it = 0; it < nmine; ++it)
+         {
+            const int s = it % kTmaStages;
+            if (it >= kTmaStages) mbar_wait(&empty[s], ((it / kTmaStages) - 1) & 1);
+            unsigned char *st = smem + (size_t)s * stage_bytes;
+            if (lane == 0 && vb)
+            {
+               mbar_expect_tx_only(&full[s], vb);
+               bulk_g2s(st, values + 4 * b0, vb, &full[s]);
+            }
+            reinterpret_cast<uint2 *>(st + cap.vbytes)[lane] = make_uint2(w0, w1);
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&full[s]);
+            if (it + 1 < nmine) scan(it + 1);
+            if (it + 2 < nmine) load(it + 2);
+         }
+      }
+      else if (lane == 0)
          for (int it = 0; it < nmine; ++it)
          {
             const int s = it % kTmaStages;
@@ -136,16 +219,18 @@ spmv_tma_kernel(int64_t row_lo, int64_t row_hi, const int64_t *__restrict__ brp,
             const int64_t n0 = row_lo + (int64_t)(first + it * stride) * R;
             const int nloc = (int)min((int64_t)R, row_hi - n0);
             const int64_t b0 = brp[n0], b1 = brp[n0 + nloc];
-            constexpr int CW = C16 ? 2 : 4;                                    // bytes per column index
-            const int64_t c0 = b0 & ~(int64_t)(16 / CW - 1), p0 = n0 & ~(int64_t)1;
             const uint32_t vb = (uint32_t)(32 * (b1 - b0));
-            const uint32_t cb = (uint32_t)((CW * (b1 - c0) + 15) & ~(int64_t)15);
-            const uint32_t pb = (uint32_t)((8 * (n0 + nloc + 1 - p0) + 15) & ~(int64_t)15);
             unsigned char *st = smem + (size_t)s * stage_bytes;
-            mbar_expect_tx(&full[s], vb + cb + pb);
-            if (vb) bulk_g2s(st, values + 4 * b0, vb, &full[s]);
-            if (cb) bulk_g2s(st + cap.vbytes, static_cast<const unsigned char *>(bcol_any) + CW * c0, cb, &full[s]);
-            bulk_g2s(st + cap.vbytes + cap.cbytes, brp + p0, pb, &full[s]);
+            {
+               constexpr int CW = COLS == kC16 ? 2 : 4;                            // bytes per column index
+               const int64_t c0 = b0 & ~(int64_t)(16 / CW - 1), p0 = n0 & ~(int64_t)1;
+               const uint32_t cb = (uint32_t)((CW * (b1 - c0) + 15) & ~(int64_t)15);
+               const uint32_t pb = (uint32_t)((8 * (n0 + nloc + 1 - p0) + 15) & ~(int64_t)15);
+               mbar_expect_tx(&full[s], vb + cb + pb);
+               if (vb) bulk_g2s(st, values + 4 * b0, vb, &full[s]);
+               if (cb) bulk_g2s(st + cap.vbytes, static_cast<const unsigned char *>(bcol_any) + CW * c0, cb, &full[s]);
+               bulk_g2s(st + cap.vbytes + cap.cbytes, brp + p0, pb, &full[s]);
+            }
          }
    }
    else
@@ -160,24 +245,43 @@ spmv_tma_kernel(int64_t row_lo, int64_t row_hi, const int64_t *__restrict__ brp,
          const int nloc = (int)min((int64_t)R, row_hi - n0);
          const unsigned char *st = smem + (size_t)s * stage_bytes;
          const double2 *sval = reinterpret_cast<const double2 *>(st);
-         using col_t = typename std::conditional<C16, int16_t, int32_t>::type;
-         const col_t *scol = reinterpret_cast<const col_t *>(st + cap.vbytes);
-         const int64_t *sbrp = reinterpret_cast<const int64_t *>(st + cap.vbytes + cap.cbytes) + (n0 & 1);
+         using col_t = typename std::conditional<COLS == kC32, int32_t, int16_t>::type;
          mbar_wait(&full[s], (it / kTmaStages) & 1);
-         const int64_t b0 = sbrp[0];
-         const int coff = (int)(b0 & (C16 ? 7 : 3));
+         const col_t *scol = nullptr;
+         const int64_t *sbrp = nullptr;
+         int coff = 0;
+         int64_t b0 = 0;
+         if constexpr (COLS != kStencil)
+         {
+            scol = reinterpret_cast<const col_t *>(st + cap.vbytes);
+            sbrp = reinterpret_cast<const int64_t *>(st + cap.vbytes + cap.cbytes) + (n0 & 1);
+            b0 = sbrp[0];
+            coff = (int)(b0 & (COLS == kC16 ? 7 : 3));
+         }
 #pragma unroll
          for (int pass = 0; pass < R * kSpmvLanes / kTmaConsumers; ++pass)
          {
             const int i = pass * (kTmaConsumers / kSpmvLanes) + tid / kSpmvLanes;
+            int pb, deg;
+            const col_t *cols;
+            if constexpr (COLS == kStencil)
+            {
+               const uint32_t w = i < nloc ? reinterpret_cast<const uint32_t *>(st + cap.vbytes)[i] : 0u;  // offset | id << 16
+               pb = (int)(w & 0xffffu);
+               cols = sdict + (w >> 16) * kDictStride;
+               deg = cols[kStencilD];
+            }
+            else
+            {
+               pb = i < nloc ? (int)(sbrp[i] - b0) : 0;
+               deg = i < nloc ? (int)(sbrp[i + 1] - b0) - pb : 0;
+               cols = scol + coff + pb;
+            }
             double y0 = 0., y1 = 0.;
             if (i < nloc)
             {
-               const int pb = (int)(sbrp[i] - b0);
-               const int deg = (int)(sbrp[i + 1] - b0) - pb;
                const double2 *row0 = sval + 2 * pb, *row1 = row0 + deg;
-               const col_t *cols = scol + coff + pb;
-               const double2 *xr = C16 ? x2 + (n0 + i) : x2;  // 16-bit indices are offsets from the row's node
+               const double2 *xr = COLS != kC32 ? x2 + (n0 + i) : x2;  // 16-bit offsets and stencils are relative to the row's node
                int t = sub;
                for (; t + 2 * kSpmvLanes < deg; t += 3 * kSpmvLanes)
                {
@@ -238,7 +342,7 @@ __global__ void diag_kernel(int64_t nnodes, const int64_t *__restrict__ brp, con
    reinterpret_cast<double2 *>(diag)[I] = d;
 }
 
-template <bool DOT, int R, int S, int L, bool C16>
+template <bool DOT, int R, int S, int L, int COLS>
 static int spmv_tma_launch(const femb200_plan *p, const RowRange &rr, const double *d_values, const double *d_x,
                            double *d_y, const double *d_flag, double *d_dot_out, bool accumulate, cudaStream_t st)
 {
@@ -247,30 +351,49 @@ static int spmv_tma_launch(const femb200_plan *p, const RowRange &rr, const doub
    const int64_t nrows = rr.hi - rr.lo;
    const int ntiles = (int)cdiv(nrows, R);
    const int maxb = rr.tile_max[R == 32 ? 0 : 1];
+   // The stages of the index layout (the 16-bit one for stencils) size the grid and decide the fall-back: the stencil
+   // mode runs the same CTAs over the same tiles as the 16-bit mode, so that the per-CTA dot partials agree bit for bit.
    SpmvTile cap;
    cap.vbytes = 32 * maxb;
-   cap.cbytes = C16 ? ((2 * (maxb + 8) + 15) & ~15) : ((4 * (maxb + 4) + 15) & ~15);
+   cap.cbytes = COLS != kC32 ? ((2 * (maxb + 8) + 15) & ~15) : ((4 * (maxb + 4) + 15) & ~15);
    cap.pbytes = ((8 * (R + 3) + 15) & ~15);
-   const size_t smem = (size_t)S * (cap.vbytes + cap.cbytes + cap.pbytes);
+   size_t smem = (size_t)S * (cap.vbytes + cap.cbytes + cap.pbytes);
    const size_t budget = devinfo().smem_optin ? devinfo().smem_optin : 227 * 1024;
    if (smem > budget) return -1;  // caller falls back to the direct kernel
-   if (int rc = ensure_dynamic_smem<spmv_tma_kernel<DOT, R, S, L, C16>>(smem)) return rc;
    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(7, (budget + 1024) / (smem + 1024)));
    const unsigned grid = (unsigned)std::min<int64_t>(ntiles, (int64_t)devinfo().sm_count * per_sm);
+   SpmvStencils dict{nullptr, nullptr, nullptr, 0};
+   if (COLS == kStencil)
+   {  // S stages of values + one word per row (value offset | id << 16), then the dictionary
+      cap.cbytes = 4 * R;
+      cap.pbytes = 0;
+      dict = SpmvStencils{p->sig, p->stencil_off, p->stencil_deg, p->nstencils};
+      smem = (size_t)S * (cap.vbytes + cap.cbytes) + ((2 * kDictStride * dict.k + 15) & ~15);
+   }
+   if (int rc = ensure_dynamic_smem<spmv_tma_kernel<DOT, R, S, L, COLS>>(smem)) return rc;
    ReduceScratch red{nullptr, nullptr};
    if (DOT)
       if (int rc = reduce_scratch(grid, st, &red)) return rc;
-   spmv_tma_kernel<DOT, R, S, L, C16><<<grid, kTmaThreads, smem, st>>>(
-       rr.lo, rr.hi, p->brp, C16 ? static_cast<const void *>(p->bcol16) : static_cast<const void *>(p->bcol), d_values, d_x, d_y,
-       d_flag, red, d_dot_out, cap, ntiles, accumulate);
+   spmv_tma_kernel<DOT, R, S, L, COLS><<<grid, kTmaThreads, smem, st>>>(
+       rr.lo, rr.hi, p->brp, COLS == kC16 ? static_cast<const void *>(p->bcol16) : static_cast<const void *>(p->bcol), dict,
+       d_values, d_x, d_y, d_flag, red, d_dot_out, cap, ntiles, accumulate);
    FEMB_LAUNCH_CHECK();
    return 0;
 }
 
+template <int COLS>
+static int spmv_tma_dispatch(const femb200_plan *p, const RowRange &rr, const double *d_values, const double *d_x,
+                             double *d_y, const double *d_flag, double *d_dot_out, bool accumulate, cudaStream_t st)
+{
+   return d_dot_out ? spmv_tma_launch<true, 64, 2, 4, COLS>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st)
+                    : spmv_tma_launch<false, 64, 2, 4, COLS>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st);
+}
+
 // y = A x on the node rows of rr (+ d_dot_out (+)= <x, y> over those rows; no-op when *d_flag != 0).
 // Default: 64-row tiles, 2 stages (3 CTAs per SM), 4 lanes per row: 0.59 ms on the n = 1448 P2 matrix against
-// 0.99 ms with 3 stages and 8 lanes (profiles/r1_summary.md).  Tiles too large for shared memory, and plans
-// with spmv_path = 1, take the direct kernel.
+// 0.99 ms with 3 stages and 8 lanes (profiles/r1_summary.md).  Columns: stencil ids when the plan has them, else
+// 16-bit offsets, else 32-bit indices (option spmv_cols forces the latter two).  Tiles too large for shared memory,
+// and plans with spmv_path = 1, take the direct kernel.
 int spmv_launch(const femb200_plan *p, const RowRange &rr, const double *d_values, const double *d_x, double *d_y,
                 const double *d_flag, double *d_dot_out, bool accumulate, cudaStream_t st)
 {
@@ -282,14 +405,13 @@ int spmv_launch(const femb200_plan *p, const RowRange &rr, const double *d_value
    }
    if (p->opt_spmv_path == 0)
    {
-      const bool c16 = p->bcol16 != nullptr && p->opt_spmv_cols != 1;
       int rc;
-      if (c16)
-         rc = d_dot_out ? spmv_tma_launch<true, 64, 2, 4, true>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st)
-                        : spmv_tma_launch<false, 64, 2, 4, true>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st);
+      if (p->sig && p->opt_spmv_cols == 0)
+         rc = spmv_tma_dispatch<kStencil>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st);
+      else if (p->bcol16 && p->opt_spmv_cols != 1)
+         rc = spmv_tma_dispatch<kC16>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st);
       else
-         rc = d_dot_out ? spmv_tma_launch<true, 64, 2, 4, false>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st)
-                        : spmv_tma_launch<false, 64, 2, 4, false>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st);
+         rc = spmv_tma_dispatch<kC32>(p, rr, d_values, d_x, d_y, d_flag, d_dot_out, accumulate, st);
       if (rc >= 0) return rc;
    }
    const unsigned grid = (unsigned)cdiv(nrows * kSpmvLanes, kSpmvThreads);

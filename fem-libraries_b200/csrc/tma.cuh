@@ -13,6 +13,11 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
 {
    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
+// raises the phase's transaction count without an arrival (the arrival follows once the thread's own stores are done)
+__device__ __forceinline__ void mbar_expect_tx_only(uint64_t *bar, uint32_t bytes)
+{
+   asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
 {
    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");

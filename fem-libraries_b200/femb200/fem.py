@@ -231,7 +231,8 @@ class Matrix:
         capi.call("femb200_plan_set_option", self._plan, key.encode(), int(value))
 
     def get_option(self, key: str) -> int:
-        """An option read back, or a read-only fact of the plan ("spmv_col_bits", "fast_records"): femb200_plan_get_option."""
+        """An option read back, or a read-only fact of the plan ("spmv_col_bits", "spmv_stencils", "fast_records"):
+        femb200_plan_get_option."""
         v = C.c_int()
         capi.call("femb200_plan_get_option", self._plan, key.encode(), C.byref(v))
         return v.value

@@ -251,7 +251,10 @@ int femb200_scatter_rows(int64_t n, int width, const int32_t *d_idx, const doubl
  * from the plan, no environment variables.
  *   "assembly_path"  0 auto | 1 visit-record kernel | 2 per-quadrature-point kernel
  *   "spmv_path"      0 auto (bulk-copy staged) | 1 direct kernel
- *   "spmv_cols"      0 auto (16-bit column offsets from the row's node when every offset of the pattern fits) | 1 32-bit
+ *   "spmv_cols"      0 auto (stencil ids: one byte per node row naming its list of column offsets in the plan's
+ *                    dictionary, when the pattern has at most 64 distinct lists of at most 32 blocks; else 16-bit
+ *                    column offsets from the row's node when every offset fits; else 32-bit) | 1 32-bit |
+ *                    2 16-bit offsets (32-bit when an offset does not fit).  Every mode gives the same y bit for bit.
  *   "vector_path"    residual vector: 0 two passes (element vectors per cell, then a gather per node) | 1 single-pass gather
  *   "prefetch_tiles" record prefetch distance of the assembly kernel in tiles (-1: 8 x SM count, 0: off)
  *   "stream_out"     0 auto (tensor bulk stores of the finished tile) | 1 store loop
@@ -259,7 +262,9 @@ int femb200_scatter_rows(int64_t n, int width, const int32_t *d_idx, const doubl
  *                    cells were damaged in the previous assembly on the plan) | 1 always | 2 never */
 int femb200_plan_set_option(femb200_plan *plan, const char *key, int value);
 /* Reads an option back, or one of the read-only facts of the plan: "spmv_col_bits" (16 or 32: the column index
- * width the staged SpMV reads with the current options), "fast_records" (1: the plan has fast-path records). */
+ * width the staged SpMV reads with the current options; 0: it reads stencil ids, no column indices), "spmv_stencils"
+ * (the number of lists in the plan's stencil dictionary, 0: the plan has none), "fast_records" (1: the plan has
+ * fast-path records). */
 int femb200_plan_get_option(const femb200_plan *plan, const char *key, int *value);
 
 /* ------------------------------------------------------------------------
