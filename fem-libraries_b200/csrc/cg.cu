@@ -345,11 +345,13 @@ namespace femb {
 // The matrix-free operator of a rank works on its whole local mesh (owned + ghost cells): the rows of the owned
 // nodes are complete, those of ghost nodes are partial and ignored, so with a partition the fused <d, A d> of the
 // apply kernel (a sum over every local node) is replaced by a dot product over the owned dofs.
+// compact: the mode of spmv_launch (0 on the matrix-free operator)
 static int cg_apply_rows(const femb200_plan *plan, int op_kind, const void *op, const double *d_values, const RowRange &rr,
-                         int64_t own_lo, int64_t own_hi, const double *d_dir, double *d_Ad, double *d_scal, cudaStream_t st)
+                         int64_t own_lo, int64_t own_hi, const double *d_dir, double *d_Ad, double *d_scal, cudaStream_t st,
+                         int compact = 0)
 {
    if (op_kind == FEMB200_OP_CSR)
-      return spmv_launch(plan, rr, d_values, d_dir, d_Ad, d_scal + SC_FLAG, d_scal + SC_RED_DEN, false, st);
+      return spmv_launch(plan, rr, d_values, d_dir, d_Ad, d_scal + SC_FLAG, d_scal + SC_RED_DEN, false, st, compact);
    const femb200_pa *pa = static_cast<const femb200_pa *>(op);
    if (own_lo == 0 && 2 * own_hi == pa_num_dofs(pa))
       return pa_apply_launch(pa, d_dir, d_Ad, d_scal + SC_FLAG, d_scal + SC_RED_DEN, st, false);
@@ -369,16 +371,23 @@ static int cg_apply_rows(const femb200_plan *plan, int op_kind, const void *op, 
 // transport, ncclAllReduce on the NCCL transport).  With use_graph the full iteration (update_r, scalar,
 // update_xdir, ghost update, apply + dot, scalar) is captured once into a CUDA graph cached in the
 // communicator and replayed; everything it needs (scalars, sequence numbers) lives in device memory.
+// On a plan with compact values (plan.cuh) the first apply also writes the kept blocks of this solve's values into the
+// plan's compact copy and checks the dropped ones; the applies of the loop then stream the copy (about a quarter fewer
+// bytes on P2), or the CSR values when a dropped block was not zero.  Both give the same bits.  The copy belongs to
+// the plan: solves on one plan must not run concurrently.
 int cg_core(const CgProblem &P, int *iters, double *final_norm, int *converged, cudaStream_t st)
 {
    const int64_t o = 2 * P.own_lo, n = 2 * (P.own_hi - P.own_lo);
    const double *dinv_o = P.dinv ? P.dinv + o : nullptr;
    double *scal = P.scal;
-   RowRange rr{0, 0, {0, 0}};
+   RowRange rr{0, 0, {0, 0}, 0};
+   int compact = 0;
    if (P.op_kind == FEMB200_OP_CSR)
    {
       FEMB_CHECK(P.plan && P.values, "pcg: the CSR operator needs a plan and values");
       if (int rc = plan_row_range(P.plan, P.own_lo, P.own_hi, &rr)) return rc;
+      femb200_plan *pm = const_cast<femb200_plan *>(P.plan);
+      compact = spmv_compact_ready(pm, rr) ? 2 : 0;
    }
    else
       FEMB_CHECK(P.op_kind == FEMB200_OP_PA && P.op, "pcg: unknown operator kind %d", P.op_kind);
@@ -393,9 +402,9 @@ int cg_core(const CgProblem &P, int *iters, double *final_norm, int *converged, 
       FEMB_LAUNCH_CHECK();
       return 0;
    };
-   auto apply = [&](cudaStream_t s) -> int {
+   auto apply = [&](cudaStream_t s, int cmode) -> int {
       if (int e = dist_halo_arena(P.comm, s)) return e;
-      if (int e = cg_apply_rows(P.plan, P.op_kind, P.op, P.values, rr, P.own_lo, P.own_hi, P.d, P.z, scal, s)) return e;
+      if (int e = cg_apply_rows(P.plan, P.op_kind, P.op, P.values, rr, P.own_lo, P.own_hi, P.d, P.z, scal, s, cmode)) return e;
       return scalar(1, SC_RED_DEN, s);
    };
    auto update_r = [&](cudaStream_t s) -> int {
@@ -417,14 +426,15 @@ int cg_core(const CgProblem &P, int *iters, double *final_norm, int *converged, 
    auto full_iteration = [&](cudaStream_t s) -> int {
       if (int e = update_r(s)) return e;
       if (int e = update_xdir(s, 0)) return e;
-      return apply(s);
+      return apply(s, compact);
    };
 
    if ((rc = femb200_cg_set_tolerances(scal, P.rtol, P.atol, st))) return rc;
    cg_init_kernel<<<gi, kVecThreads, 0, st>>>(n, P.b + o, dinv_o, P.x + o, P.r + o, P.d + o, red, scal + SC_RED_NOM);
    FEMB_LAUNCH_CHECK();
    if ((rc = scalar(0, SC_RED_NOM, st))) return rc;
-   if ((rc = apply(st))) return rc;
+   if (compact) FEMB_CUDA(cudaMemsetAsync(P.plan->cbad, 0, sizeof(int), st));
+   if ((rc = apply(st, compact ? 1 : 0))) return rc;
 
    const int nit = P.fixed_iters > 0 ? P.fixed_iters : P.maxit;
    const int check_every = P.check_every > 0 ? P.check_every : 25;
@@ -442,7 +452,7 @@ int cg_core(const CgProblem &P, int *iters, double *final_norm, int *converged, 
       else if (G && i >= 2)
       {  // iteration 1 ran eagerly (warm kernels, NCCL connections); capture on first use, then replay
          const void *key[8] = {P.plan, P.op, P.values, P.x, P.r, P.d, P.z, P.dinv};
-         const int64_t ikey[3] = {P.own_lo, P.own_hi, (int64_t)P.op_kind};
+         const int64_t ikey[4] = {P.own_lo, P.own_hi, (int64_t)P.op_kind, (int64_t)compact};
          if (!G->exec || memcmp(G->key, key, sizeof(key)) || memcmp(G->ikey, ikey, sizeof(ikey)))
          {
             if (G->exec) cudaGraphExecDestroy(G->exec), G->exec = nullptr;
@@ -497,7 +507,7 @@ extern "C" int femb200_cg_apply(const femb200_plan *plan, int op_kind, const voi
                                 const double *d_dir, double *d_Ad, double *d_scal, void *stream)
 {
    FEMB_CHECK(d_dir && d_Ad && d_scal, "cg_apply: null argument");
-   RowRange rr{0, 0, {0, 0}};
+   RowRange rr{0, 0, {0, 0}, 0};
    if (op_kind == FEMB200_OP_CSR)
    {
       FEMB_CHECK(plan && d_values, "cg_apply: CSR operator needs a plan and values");

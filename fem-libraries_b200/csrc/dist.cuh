@@ -89,7 +89,7 @@ struct IterGraph
 {
    cudaGraphExec_t exec = nullptr;
    const void *key[8] = {};
-   int64_t ikey[3] = {};
+   int64_t ikey[4] = {};
 };
 IterGraph *dist_iter_graph(femb200_dist *D);
 cudaStream_t dist_capture_stream(femb200_dist *D);

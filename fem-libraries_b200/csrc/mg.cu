@@ -1004,7 +1004,7 @@ extern "C" int femb200_pcg_mg(femb200_mg *mg, const double *d_b, double *d_x, do
    const MgLevel &f = mg->lev[0];
    const int64_t n = f.n, n2 = n / 2;
    double *r = d_work, *d = d_work + n, *z = d_work + 2 * n, *Ad = d_work + 3 * n, *scal = d_work + 4 * n;
-   RowRange rr{0, 0, {0, 0}};
+   RowRange rr{0, 0, {0, 0}, 0};
    if (f.plan)
       if (int rc = plan_row_range(f.plan, 0, f.nnodes, &rr)) return rc;
    const unsigned grid = mg_grid(n2);

@@ -10,6 +10,8 @@
 //     rowptr[2I]   = 4 brp[I]
 //     rowptr[2I+1] = 4 brp[I] + 2 deg(I)
 //     colidx[rowptr[2I+i] + 2s + k] = 2 bcol[brp[I]+s] + k
+#include <vector>
+
 #include "plan.cuh"
 
 namespace femb {
@@ -716,6 +718,168 @@ done:
    return 0;
 }
 
+// --- compact values of the PCG (plan.cuh) ------------------------------------------------
+// keep[I] bit s: some cell holds node I and the column of slot s other than as a vertex / opposite-edge pair (P2,
+// basix order: edge 3 + i is opposite vertex i); the slots left unmarked are the dropped blocks.  flags[0]: a column
+// is missing from its row's stencil.
+__global__ void k_compact_mark(int64_t ncells, const int32_t *__restrict__ dofmap, const uint8_t *__restrict__ sig,
+                               const int16_t *__restrict__ off, const uint8_t *__restrict__ sdeg, uint32_t *__restrict__ keep,
+                               int32_t *__restrict__ flags)
+{
+   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+   if (e >= ncells) return;
+   int32_t d[6];
+#pragma unroll
+   for (int a = 0; a < 6; ++a) d[a] = dofmap[6 * e + a];
+   for (int a = 0; a < 6; ++a)
+   {
+      const int id = sig[d[a]], deg = sdeg[id];
+      uint32_t m = 0;
+      for (int b = 0; b < 6; ++b)
+      {
+         if (b == a + 3 || a == b + 3) continue;
+         const int o = d[b] - d[a];
+         int s = 0;
+         while (s < deg && off[id * kStencilD + s] != o) ++s;
+         if (s == deg)
+            atomicOr(flags, 1);
+         else
+            m |= 1u << s;
+      }
+      atomicOr(keep + d[a], m);
+   }
+}
+
+__device__ __forceinline__ unsigned long long compact_key(int id, uint32_t keep)
+{
+   return ((unsigned long long)(id + 1) << 32) | keep;  // never 0 (the empty slot)
+}
+
+// open-addressing table of the distinct (stencil id, kept mask) keys; flags[0] when it overflows
+__global__ void k_compact_insert(int64_t nnodes, const uint8_t *__restrict__ sig, const uint32_t *__restrict__ keep,
+                                 unsigned long long *keys, int32_t *flags)
+{
+   const int64_t I = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+   if (I >= nnodes) return;
+   const unsigned long long h = compact_key(sig[I], keep[I]);
+   unsigned s = (unsigned)((h * 0x9e3779b97f4a7c15ull) >> 54) & (kStencilH - 1);
+   for (int probe = 0; probe < kStencilH; ++probe, s = (s + 1) & (kStencilH - 1))
+   {
+      unsigned long long k = *(volatile unsigned long long *)&keys[s];
+      if (k == 0) k = atomicCAS(&keys[s], 0ull, h);
+      if (k == 0 || k == h) return;
+   }
+   atomicOr(flags, 1);
+}
+
+// csig[I] = the row's key number (ids[table slot]); kept[I] = its kept degree (scanned into cbrp)
+__global__ void k_compact_assign(int64_t nnodes, const uint8_t *__restrict__ sig, const uint32_t *keep,
+                                 const unsigned long long *__restrict__ keys, const int32_t *__restrict__ ids,
+                                 uint8_t *__restrict__ csig, int32_t *kept)  // kept aliases keep
+{
+   const int64_t I = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+   if (I >= nnodes) return;
+   const uint32_t m = keep[I];
+   const unsigned long long h = compact_key(sig[I], m);
+   unsigned s = (unsigned)((h * 0x9e3779b97f4a7c15ull) >> 54) & (kStencilH - 1);
+   while (keys[s] != h) s = (s + 1) & (kStencilH - 1);  // every key was inserted
+   csig[I] = (uint8_t)ids[s];
+   kept[I] = __popc(m);
+}
+
+// Compact keys of the node rows (plan.cuh), P2 plans with a stencil dictionary.  Leaves p->csig null (no compact
+// values) when a column is missing from a stencil, there are more than kCompactK keys or no block is dropped.
+static int plan_compact(femb200_plan *p, cudaStream_t st)
+{
+   const int64_t nnodes = p->nnodes;
+   const int T = 256;
+   unsigned char *scratch = nullptr;  // keys [H] u64 | ids [H] | flags | keep [nnodes] (then the kept degrees)
+   const size_t head = kStencilH * (8 + 4) + 16;
+   FEMB_CUDA(cudaMalloc(&scratch, head + 4 * ((size_t)nnodes + 1)));
+   auto *keys = reinterpret_cast<unsigned long long *>(scratch);
+   auto *ids = reinterpret_cast<int32_t *>(scratch + 8 * kStencilH), *flags = ids + kStencilH;
+   auto *keep = reinterpret_cast<uint32_t *>(scratch + head);
+   std::vector<unsigned long long> hkeys(kStencilH);
+   std::vector<int32_t> hids(kStencilH, 0);
+   std::vector<int16_t> hoff(kStencilK * kStencilD), hdict;
+   std::vector<uint8_t> hdeg(kStencilK);
+   int32_t bad = 0;
+   int nkeys = 0;
+   bool dropped = false;
+   size_t bytes = 0;
+   int rc = 0;
+   cudaMemsetAsync(scratch, 0, head + 4 * (size_t)nnodes, st);
+   k_compact_mark<<<(unsigned)cdiv(p->ncells, T), T, 0, st>>>(p->ncells, p->dofmap, p->sig, p->stencil_off, p->stencil_deg,
+                                                              keep, flags);
+   k_compact_insert<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, p->sig, keep, keys, flags);
+   if (cudaMemcpyAsync(hkeys.data(), keys, 8 * kStencilH, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+       cudaMemcpyAsync(&bad, flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+       cudaMemcpyAsync(hoff.data(), p->stencil_off, 2 * hoff.size(), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+       cudaMemcpyAsync(hdeg.data(), p->stencil_deg, hdeg.size(), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+       cudaStreamSynchronize(st) != cudaSuccess)
+   {
+      rc = set_error("plan_create: compact keys failed: %s", cudaGetErrorString(cudaGetLastError()));
+      goto done;
+   }
+   for (int s = 0; s < kStencilH && !bad; ++s)
+   {
+      if (!hkeys[s]) continue;
+      if (nkeys == kCompactK)
+      {
+         bad = 1;
+         break;
+      }
+      hids[s] = nkeys++;
+      const int id = (int)(hkeys[s] >> 32) - 1, deg = hdeg[id];
+      const uint32_t m = (uint32_t)hkeys[s];
+      const size_t e = hdict.size();
+      hdict.resize(e + kCDictStride, 0);
+      int c = 0;
+      for (int t = 0; t < kStencilD; ++t) hdict[e + t] = hoff[id * kStencilD + t];
+      for (int t = 0; t < kStencilD; ++t)
+      {
+         const bool kept = t < deg && ((m >> t) & 1u);
+         hdict[e + kStencilD + 2 + t] = kept ? (int16_t)c++ : (int16_t)-1;
+         dropped |= t < deg && !kept;
+      }
+      hdict[e + kStencilD] = (int16_t)deg, hdict[e + kStencilD + 1] = (int16_t)c;
+   }
+   if (bad || !dropped) goto done;
+   if ((rc = dev_alloc(&p->csig, (size_t)nnodes, &bytes)) || (rc = dev_alloc(&p->cdict, hdict.size(), &bytes)) ||
+       (rc = dev_alloc(&p->cbrp, (size_t)nnodes + 1, &bytes)))
+      goto done;
+   if (cudaMemcpyAsync(ids, hids.data(), 4 * kStencilH, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+       cudaMemcpyAsync(p->cdict, hdict.data(), 2 * hdict.size(), cudaMemcpyHostToDevice, st) != cudaSuccess)
+   {
+      rc = set_error("plan_create: compact dictionary upload failed");
+      goto done;
+   }
+   k_compact_assign<<<(unsigned)cdiv(nnodes, T), T, 0, st>>>(nnodes, p->sig, keep, keys, ids, p->csig,
+                                                             reinterpret_cast<int32_t *>(keep));
+   if ((rc = exclusive_scan_i32_i64(reinterpret_cast<int32_t *>(keep), p->cbrp, nnodes, st))) goto done;
+   {
+      int32_t *tmax = flags;
+      cudaMemsetAsync(tmax, 0, sizeof(int32_t), st);
+      k_range_tile_max<<<(unsigned)cdiv(cdiv(nnodes, 64), T), T, 0, st>>>(0, nnodes, 64, p->cbrp, tmax);
+      if (cudaMemcpyAsync(&p->nkept, p->cbrp + nnodes, sizeof(int64_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+          cudaMemcpyAsync(&p->ctile_max, tmax, sizeof(int32_t), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+          cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess)
+         rc = set_error("plan_create: compact row pointer failed: %s", cudaGetErrorString(cudaGetLastError()));
+   }
+done:
+   cudaFree(scratch);
+   if (rc || !p->cbrp)
+   {
+      cudaFree(p->csig), cudaFree(p->cdict), cudaFree(p->cbrp);
+      p->csig = nullptr, p->cdict = nullptr, p->cbrp = nullptr;
+      p->nkept = 0, p->ctile_max = 0;
+      return rc;
+   }
+   p->ncompact = nkeys;
+   p->bytes += bytes;
+   return 0;
+}
+
 }  // namespace femb
 
 using namespace femb;
@@ -736,6 +900,11 @@ extern "C" void femb200_plan_destroy(femb200_plan *p)
    cudaFree(p->sig);
    cudaFree(p->stencil_off);
    cudaFree(p->stencil_deg);
+   cudaFree(p->csig);
+   cudaFree(p->cdict);
+   cudaFree(p->cbrp);
+   cudaFree(p->cvalues);
+   cudaFree(p->cbad);
    cudaFree(p->dslot);
    cudaFree(p->bc);
    cudaFree(p->bc_nodes);
@@ -845,6 +1014,7 @@ extern "C" int femb200_plan_create(int etype, int64_t nnodes, int64_t ncells, co
       cudaMemsetAsync(flags, 0, sizeof(int32_t) * 2, st);
    }
    if (p->bcol16 && (rc = plan_stencils(p, st))) return fail(rc);
+   if (etype == FEMB200_P2 && p->sig && (rc = plan_compact(p, st))) return fail(rc);
 
    // 3. slot map + staging-tile sizes
    k_fill_slots<<<(unsigned)cdiv(nnodes, 128), 128, 0, st>>>(nnodes, nd, tri, d_dofmap, p->nptr, tmpvis, p->brp, p->bcol,
@@ -1056,27 +1226,29 @@ int plan_row_range(const femb200_plan *p, int64_t lo, int64_t hi, RowRange *out)
               (long long)hi, (long long)p->nnodes);
    out->lo = lo, out->hi = hi;
    out->tile_max[0] = p->tile_max_blocks[0], out->tile_max[1] = p->tile_max_blocks[1];
+   out->ctile_max = p->ctile_max;
    if (lo % 64 == 0 || hi == lo) return 0;
    femb200_plan *pm = const_cast<femb200_plan *>(p);
    std::lock_guard<std::mutex> lock(pm->range_mtx);
    auto it = pm->range_tile_max.find(std::make_pair(lo, hi));
    if (it == pm->range_tile_max.end())
    {
-      int32_t *d = nullptr, h[2] = {0, 0};
-      FEMB_CUDA(cudaMalloc(&d, 2 * sizeof(int32_t)));
-      FEMB_CUDA(cudaMemset(d, 0, 2 * sizeof(int32_t)));
-      for (int k = 0; k < 2; ++k)
+      int32_t *d = nullptr, h[3] = {0, 0, 0};
+      FEMB_CUDA(cudaMalloc(&d, 3 * sizeof(int32_t)));
+      FEMB_CUDA(cudaMemset(d, 0, 3 * sizeof(int32_t)));
+      for (int k = 0; k < 3; ++k)
       {
-         const int R = 32 << k;
+         const int R = k == 0 ? 32 : 64;
          const int64_t nt = cdiv(hi - lo, R);
-         k_range_tile_max<<<(unsigned)cdiv(nt, 256), 256>>>(lo, hi, R, p->brp, d + k);
+         if (k < 2 || p->cbrp) k_range_tile_max<<<(unsigned)cdiv(nt, 256), 256>>>(lo, hi, R, k < 2 ? p->brp : p->cbrp, d + k);
       }
       const cudaError_t e = cudaMemcpy(h, d, sizeof(h), cudaMemcpyDeviceToHost);
       cudaFree(d);
       FEMB_CHECK(e == cudaSuccess, "row range: %s", cudaGetErrorString(e));
-      it = pm->range_tile_max.emplace(std::make_pair(lo, hi), std::array<int32_t, 2>{h[0], h[1]}).first;
+      it = pm->range_tile_max.emplace(std::make_pair(lo, hi), std::array<int32_t, 3>{h[0], h[1], h[2]}).first;
    }
    out->tile_max[0] = it->second[0], out->tile_max[1] = it->second[1];
+   out->ctile_max = it->second[2];
    return 0;
 }
 }  // namespace femb
@@ -1118,6 +1290,11 @@ extern "C" int femb200_plan_set_option(femb200_plan *p, const char *key, int val
                  "plan_set_option: spmv_cols must be 0 (auto: stencil ids, else 16-bit offsets), 1 (32-bit) or 2 (16-bit offsets)");
       p->opt_spmv_cols = value;
    }
+   else if (!strcmp(key, "spmv_compact"))
+   {
+      FEMB_CHECK(value == 0 || value == 1, "plan_set_option: spmv_compact must be 0 (auto: compact values in PCG) or 1 (off)");
+      p->opt_spmv_compact = value;
+   }
    else if (!strcmp(key, "vector_path"))
    {
       FEMB_CHECK(value == 0 || value == 1, "plan_set_option: vector_path must be 0 (two passes) or 1 (single-pass gather)");
@@ -1157,6 +1334,10 @@ extern "C" int femb200_plan_get_option(const femb200_plan *p, const char *key, i
       *value = (p->sig && p->opt_spmv_cols == 0) ? 0 : (p->bcol16 && p->opt_spmv_cols != 1) ? 16 : 32;
    else if (!strcmp(key, "spmv_stencils"))
       *value = p->sig ? p->nstencils : 0;
+   else if (!strcmp(key, "spmv_compact"))
+      *value = p->opt_spmv_compact;
+   else if (!strcmp(key, "spmv_compact_keys"))
+      *value = p->csig ? p->ncompact : 0;
    else if (!strcmp(key, "fast_records"))
       *value = p->frec ? 1 : 0;
    else

@@ -104,6 +104,13 @@ constexpr int kNumTileR = 6;
 // kStencilK lists of at most kStencilD offsets (a lattice numbering has a handful: 16 for P2 triangles).
 constexpr int kStencilK = 64;
 constexpr int kStencilD = 32;
+// Compact values of the PCG (P2 triangles with a stencil dictionary): the blocks of a vertex and the midpoint of the
+// opposite edge are zero on every straight-sided cell (their gradient products integrate (4 l_a - 1) l_b to 0), and no
+// other cell holds that pair.  A compact key = (stencil id, mask of the kept slots); its dictionary entry holds, in
+// int16 words: the stencil's column offsets [kStencilD], the degree, the kept degree, and per slot its position in the
+// compact row or -1 when the block is dropped [kStencilD].  33 words per entry: keys start in different banks.
+constexpr int kCompactK = 64;
+constexpr int kCDictStride = 2 * kStencilD + 2;
 __host__ __device__ constexpr int tile_r(int r) { return r == 0 ? 32 : r == 1 ? 64 : r == 2 ? 96 : r == 3 ? 128 : r == 4 ? 192 : 256; }
 
 }  // namespace femb
@@ -130,6 +137,17 @@ struct femb200_plan
    int16_t *stencil_off = nullptr;                        // [nstencils][kStencilD] offsets, in the plan's column order
    uint8_t *stencil_deg = nullptr;                        // [nstencils] block degree of each stencil
    int32_t nstencils = 0;
+   // compact values of the PCG (plan.cuh above; null / 0 when the plan has none): the kept blocks of row I are
+   // cvalues[4 cbrp[I], 4 cbrp[I + 1]) in the scalar-row layout of the CSR (kept row-0 halves, then row-1 halves)
+   uint8_t *csig = nullptr;        // [nnodes] compact key of each node row
+   int16_t *cdict = nullptr;       // [ncompact][kCDictStride]
+   int64_t *cbrp = nullptr;        // [nnodes+1] first kept block of each node row
+   int32_t ncompact = 0;
+   int64_t nkept = 0;
+   int32_t ctile_max = 0;          // kept blocks of the largest 64-row tile (tiles aligned to 64 rows)
+   double *cvalues = nullptr;      // [4 nkept] allocated by the first solve that uses it (cg.cu), then kept
+   int *cbad = nullptr;            // device word: set by a solve's first apply when a dropped block is not +-0
+   bool cvalues_failed = false;    // the allocation failed once: solves take the full path
    uint8_t *dslot = nullptr;                              // [nnodes] slot of the diagonal block in its row (255: none)
    int32_t tile_max_blocks[femb::kNumTileR] = {0, 0, 0, 0, 0, 0};
    // Dirichlet
@@ -162,11 +180,13 @@ struct femb200_plan
    int opt_assembly_path = 0;    // 0 auto; 1 visit-record kernel; 2 per-quadrature-point kernel
    int opt_spmv_path = 0;        // 0 auto (bulk-copy staged, persistent); 1 direct kernel
    int opt_spmv_cols = 0;        // 0 auto (stencil ids, else 16-bit relative indices, else 32-bit); 1 32-bit; 2 16-bit
+   int opt_spmv_compact = 0;     // 0 auto (PCG applies stream the compact values when the plan has them); 1 off
    int opt_vector_path = 0;      // residual vector: 0 two passes (per-cell r_e + gather); 1 single-pass gather
    int opt_prefetch_tiles = -1;  // record prefetch distance of the assembly kernel in tiles (-1: 8 x SM count)
-   // largest 32- / 64-row SpMV tile (in node blocks) of the tiling that starts at row_lo, per row range
-   // [row_lo, row_hi) that has been applied (the owned rows of a rank; measured once, on first use)
-   std::map<std::pair<int64_t, int64_t>, std::array<int32_t, 2>> range_tile_max;
+   // largest 32- / 64-row SpMV tile (in node blocks) of the tiling that starts at row_lo, then the largest 64-row tile
+   // of the compact values, per row range [row_lo, row_hi) that has been applied (the owned rows of a rank; measured
+   // once, on first use)
+   std::map<std::pair<int64_t, int64_t>, std::array<int32_t, 3>> range_tile_max;
    std::mutex range_mtx;
 };
 
@@ -176,6 +196,7 @@ struct RowRange
 {
    int64_t lo, hi;
    int32_t tile_max[2];
+   int32_t ctile_max;  // largest 64-row tile of the compact values (0: the plan has none)
 };
 // builds p->cref / allocates p->tdam for a record stage of `cap` cells per tile and writes the slot numbers into the
 // fast records
@@ -186,6 +207,11 @@ int plan_row_range(const femb200_plan *p, int64_t lo, int64_t hi, RowRange *out)
 inline size_t plan_cell_scratch_doubles(int etype) { return etype == FEMB200_P1 ? 12 : 24; }
 // allocates p->celld on first use
 int plan_cell_scratch(femb200_plan *p);
+// compact: 0 the CSR values; 1 the CSR values, and the kept blocks are written to p->cvalues (a dropped block that is
+// not +-0 sets *p->cbad); 2 the compact values when *p->cbad == 0, else the CSR values (switched on the device).
 int spmv_launch(const femb200_plan *p, const RowRange &rr, const double *d_values, const double *d_x, double *d_y,
-                const double *d_flag, double *d_dot_out, bool accumulate, cudaStream_t st);
+                const double *d_flag, double *d_dot_out, bool accumulate, cudaStream_t st, int compact = 0);
+// true when the PCG applies of rr can use the compact values (option, plan, stage sizes); allocates p->cvalues and
+// p->cbad on first use and returns false when that fails
+bool spmv_compact_ready(femb200_plan *p, const RowRange &rr);
 }  // namespace femb

@@ -226,13 +226,14 @@ class Matrix:
         self._bc_marker = m
 
     def set_option(self, key: str, value: int):
-        """Kernel selection of the plan (femb200_plan_set_option): "assembly_path", "spmv_path", "spmv_cols", "vector_path", "prefetch_tiles",
+        """Kernel selection of the plan (femb200_plan_set_option): "assembly_path", "spmv_path", "spmv_cols", "spmv_compact"
+        (0: PCG applies stream the compact values where the plan has them, 1: off), "vector_path", "prefetch_tiles",
         "stream_out", "damage_stage"."""
         capi.call("femb200_plan_set_option", self._plan, key.encode(), int(value))
 
     def get_option(self, key: str) -> int:
-        """An option read back, or a read-only fact of the plan ("spmv_col_bits", "spmv_stencils", "fast_records"):
-        femb200_plan_get_option."""
+        """An option read back, or a read-only fact of the plan ("spmv_col_bits", "spmv_stencils", "spmv_compact_keys",
+        "fast_records"): femb200_plan_get_option."""
         v = C.c_int()
         capi.call("femb200_plan_get_option", self._plan, key.encode(), C.byref(v))
         return v.value

@@ -255,6 +255,14 @@ int femb200_scatter_rows(int64_t n, int width, const int32_t *d_idx, const doubl
  *                    dictionary, when the pattern has at most 64 distinct lists of at most 32 blocks; else 16-bit
  *                    column offsets from the row's node when every offset fits; else 32-bit) | 1 32-bit |
  *                    2 16-bit offsets (32-bit when an offset does not fit).  Every mode gives the same y bit for bit.
+ *   "spmv_compact"   0 auto | 1 off.  Auto: on a P2 plan with compact keys (see below) the operator applies inside
+ *                    femb200_pcg / femb200_dist_pcg stream a copy of the values without the vertex / opposite-edge
+ *                    blocks (zero on every straight-sided cell), about a quarter fewer bytes.  The first apply of each
+ *                    solve writes the copy from that solve's values and checks that every dropped block is +-0; when
+ *                    one is not (curved or damaged cells, edited values) the solve streams the CSR values.  The copy
+ *                    (32 B per kept block) is allocated by the first solve on the plan and shared by later ones; when
+ *                    it cannot be allocated the solves stream the CSR values.  Iterates are bit-identical either way
+ *                    (finite iterates).  Solves on one plan must not run concurrently.
  *   "vector_path"    residual vector: 0 two passes (element vectors per cell, then a gather per node) | 1 single-pass gather
  *   "prefetch_tiles" record prefetch distance of the assembly kernel in tiles (-1: 8 x SM count, 0: off)
  *   "stream_out"     0 auto (tensor bulk stores of the finished tile) | 1 store loop
@@ -263,7 +271,8 @@ int femb200_scatter_rows(int64_t n, int width, const int32_t *d_idx, const doubl
 int femb200_plan_set_option(femb200_plan *plan, const char *key, int value);
 /* Reads an option back, or one of the read-only facts of the plan: "spmv_col_bits" (16 or 32: the column index
  * width the staged SpMV reads with the current options; 0: it reads stencil ids, no column indices), "spmv_stencils"
- * (the number of lists in the plan's stencil dictionary, 0: the plan has none), "fast_records" (1: the plan has
+ * (the number of lists in the plan's stencil dictionary, 0: the plan has none), "spmv_compact_keys" (the number of
+ * (stencil, kept blocks) keys of the compact values, 0: the plan has none), "fast_records" (1: the plan has
  * fast-path records). */
 int femb200_plan_get_option(const femb200_plan *plan, const char *key, int *value);
 
